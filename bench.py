@@ -1,8 +1,13 @@
 #!/usr/bin/env python3
 """bench.py -- ECDSA verifies/s at batch 2^20 per GPU (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step returned (the verify result
+per row, 0.0 / 1.0) as DIR/ecdsa_verify_ok.npy (float32; one file per rank,
+ecdsa_verify_ok_rank<g>.npy, when N > 1).  The inputs depend only on the
+arguments, so two builds can be compared output for output.
 
 A step = one pass of the hot path (secec Verify, EncodingCompact) over one
 batch of 2^20 synthetic (public key, digest, signature) rows per GPU; rank g
@@ -153,6 +158,8 @@ def cpu_reference_arm(args):
             "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     emit(line)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"ecdsa_verify_ok": ok})
     return 0
 
 
@@ -166,6 +173,23 @@ def hbm_peak_gbs():
             return float(json.load(f)["hbm_gbs"])
     except (OSError, KeyError, ValueError):
         return 6548.2
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each 1-D array as out_dir/<name>.npy in float32.  An array too large for DUMP_BYTES is replaced by a
+    fixed, seeded sample of its rows, written with the sampled row numbers (<name>_rows.npy, float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a).reshape(-1)
+        if a.size * 4 > budget:
+            rows = np.sort(np.random.default_rng(0).choice(a.size, budget // 12, replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def emit(line):
@@ -189,7 +213,11 @@ def main():
     ap.add_argument("--headline-only", action="store_true",
                     help="only the device-resident headline steps (for the ncu launch list in profiles/): "
                          "no end-to-end leg, no other paths")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly ONE JSON line: libraries that print to the C-level stdout (NCCL's version
     # banner, for one) are sent to stderr for the duration of the run
     global _REAL_STDOUT
@@ -286,7 +314,8 @@ def main():
     ms_total = max_over_ranks(ms_total)
     ms_per_step = ms_total / args.steps
     value = n * world / (ms_per_step * 1e-3)
-    assert np.array_equal(ok.cpu().numpy(), expected)
+    ok_last = ok.cpu().numpy()
+    assert np.array_equal(ok_last, expected)
 
     # ---- end to end through the C ABI with host buffers --------------------------
     np_pk, np_dg, np_sg = h_pk.numpy(), h_dg.numpy(), h_sg.numpy()
@@ -571,6 +600,8 @@ def main():
             "input_generation_s": t_gen,
         }
         emit(line)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"ecdsa_verify_ok" + (f"_rank{rank}" if world > 1 else ""): ok_last})
     eng.close()
     if world > 1:
         dist.destroy_process_group()

@@ -40,9 +40,9 @@ CT_KERNELS = ("k_base_mult_ct", "k_scalar_mult_ct", "k_rfc6979_nonce", "k_sign_f
 
 
 def test_secret_independent_counters(tmp_path):
-    ncu = shutil.which("ncu") or "/usr/local/cuda/bin/ncu"
-    if not os.path.exists(ncu):
-        pytest.skip("ncu not installed")
+    ncu = shutil.which("ncu") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "ncu")
+    if not os.access(ncu, os.X_OK):
+        pytest.skip("Nsight Compute (ncu) is not installed or not executable here")
     log = tmp_path / "ct.csv"
     cmd = [ncu, "--metrics", ",".join(METRICS), "--clock-control", "none", "--profile-from-start", "off", "--csv",
            "--log-file", str(log), sys.executable, os.path.join(ROOT, "tests", "ct", "ct_probe.py")]
