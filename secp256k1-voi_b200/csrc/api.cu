@@ -1273,7 +1273,7 @@ extern "C" int s256_debug_ladder_add_count(s256_ctx *ctx, size_t n, uint64_t *ad
 }
 // executed MAC32 of one k_dsm item given its measured number of ladder additions (both halves) and beta multiplications
 // The Jacobian ladder (jac.cuh): doubling 2 M + 5 S (or 3 M + 4 S), mixed addition 6 M + 3 S + one fused pair, the table's
-// scaling to a common denominator (kernels.cuh) and the conversion of the result.
+// co-Z chain and its scaling to a common denominator (kernels.cuh) and the conversion of the result.
 struct dsm_costs {
     double dbl, add, mix, table, tail;
 };
@@ -1293,11 +1293,10 @@ static dsm_costs dsm_cost_model() {
 #endif
     c.mix = 6 * M + 3 * S + F2;
     c.add = c.mix;  // the ladder adds affine rows
-    // 8 doublings + 7 mixed additions; TS - 2 suffix products; per row k = 3 .. TS - 1 two products for the cofactor
-    // Z_all / Z_k and the running prefix (one for the last row), S + 3 M to scale a row, the same for P itself, and
-    // one product to come back from the isomorphic curve -- no inversion
-    c.table = (DSM_TS / 2) * c.dbl + (DSM_TS / 2 - 1) * c.mix + (DSM_TS - 2) * M + (2 * (DSM_TS - 3) + 1) * M +
-              DSM_TS * (3 * M + S) + M;
+    // co-Z chain (kernels.cuh): DBLU M + 5 S, TS - 2 ZADDU of 4 M + 2 S; the backward pass TS - 3 ratio products and
+    // 3 M + S for each of the TS - 2 rows not yet at Z_all; Z_all = 2y r_2, and one product to come back from the
+    // isomorphic curve -- no inversion
+    c.table = (M + 5 * S) + (DSM_TS - 2) * (4 * M + 2 * S) + (DSM_TS - 3) * M + (DSM_TS - 2) * (3 * M + S) + 2 * M;
     c.tail = 2 * M + S;
 #else
 #ifndef S256_NO_FUSED

@@ -48,8 +48,8 @@ S256_HD void jac_double(F &fo, pt &v, const pt &p) {
     fo.mul(f, e, t);  // Y3 = E (D - X3) - 8 C
     fo.submul8(v.y, f, c);
 }
-// v = p + (x2, y2) for a finite p whose sum with the addend is known not to be exceptional (table construction:
-// k P + P with 2 <= k < 16 on a curve of prime order).
+// v = p + (x2, y2) for a finite p whose sum with the addend is known not to be exceptional (the constant-time
+// fixed-base accumulation, whose argument is given where it is used).
 template <class F>
 S256_HD void jac_add_mixed_nocheck(F &fo, pt &v, const pt &p, const fe &x2, const fe &y2) {
     fe zz, u2, s2, h, r, hh, hhh, w, t, x3;
@@ -69,6 +69,52 @@ S256_HD void jac_add_mixed_nocheck(F &fo, pt &v, const pt &p, const fe &x2, cons
     fo.sub(t, w, x3);
     fo.mul2sub(v.y, r, t, p.y, hhh);
     v.x = x3;
+}
+
+// Co-Z formulas (Meloni 2007; Goundar, Joye, Miyaji 2011) for chains of consecutive multiples: two points kept at ONE
+// shared Z, which neither formula computes -- the caller follows it through the returned ratio.
+//
+// DBLU from an affine point P = (x, y): (x2, y2) = 2P at Z = 2y, and (x1, y1) = P at that same Z, (4 x y^2, 8 y^4),
+// which the doubling produces on the way: 1 M + 5 S.  2y != 0: there is no 2-torsion on a curve of prime order.
+template <class F>
+S256_HD void jac_dblu(F &fo, fe &x2, fe &y2, fe &x1, fe &y1, const fe &x, const fe &y) {
+    fe a, b, c, d, e, t;
+    fo.sqr(a, x);
+    fo.sqr(b, y);
+    fo.sqr(c, b);
+    fo.add(t, x, b);  // D = 2 ((x + B)^2 - A - C) = 4 x B
+    fo.sqr(t, t);
+    fo.sub(t, t, a);
+    fo.sub(t, t, c);
+    fo.mul2(d, t);
+    fo.mul3(e, a);  // E = 3 A
+    fo.sqr(t, e);
+    fo.sub2(x2, t, d);  // X = E^2 - 2 D
+    fo.sub(t, d, x2);
+    fo.mul(a, e, t);
+    fo.submul8(y2, a, c);  // Y = E (D - X) - 8 C
+    x1 = d;
+    fo.mul8(y1, c);
+}
+// ZADDU: for P = (x1, y1) and Q = (x2, y2) at one shared Z, Q becomes P + Q and P becomes P again, both at the Z of the
+// sum, which is Z u with u = x1 - x2 (returned): 4 M + 2 S.  Not for P = +-Q (u = 0) nor for either at infinity.
+template <class F>
+S256_HD void jac_zaddu(F &fo, fe &x1, fe &y1, fe &x2, fe &y2, fe &u) {
+    fe c, w1, w2, r, t;
+    fo.sub(u, x1, x2);
+    fo.sqr(c, u);
+    fo.mul(w1, x1, c);  // W1 = X1 C
+    fo.mul(w2, x2, c);  // W2 = X2 C
+    fo.sub(r, y1, y2);
+    fo.sub(t, w1, w2);
+    fo.mul(y1, y1, t);  // A1 = Y1 (W1 - W2)
+    fo.sqr(t, r);
+    fo.sub(t, t, w1);
+    fo.sub(x2, t, w2);  // X3 = (Y1 - Y2)^2 - W1 - W2
+    fo.sub(t, w1, x2);
+    fo.mul(c, r, t);
+    fo.sub(y2, c, y1);  // Y3 = (Y1 - Y2) (W1 - X3) - A1
+    x1 = w1;
 }
 
 // acc += (x2, y2), every case handled; inf is the caller's "accumulator is the identity" flag.

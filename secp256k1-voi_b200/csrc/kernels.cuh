@@ -10,7 +10,7 @@
 //   u1    sc    G-side scalar                                    32 B
 //   dig1/2 int8 [ND][n] signed window digits of the GLV halves   2*ND B
 //   sfl   u8    bit0 scalars-valid, bit1 negate P, bit2 negate lambda*P
-//   tbl   pt    [TS] multiples 1..TS of P (projective)           96*TS B
+//   tbl   pt    multiples 1..TS of P (see item_dsm_table)        96*DSM_TSTRIDE B
 //   res   pt    projective result                                96 B
 #pragma once
 #include "fe.cuh"
@@ -30,12 +30,12 @@ constexpr int DSM_ND = glv_recode<DSM_W>::ND;  // digits per 128-bit half
 constexpr int DSM_TS = 1 << (DSM_W - 1);       // table entries 1..TS
 // The verification ladder runs in Jacobian coordinates over an AFFINE per-item table (jac.cuh) unless S256_DSM_RCB
 // asks for the round-1 form (complete projective formulas, projective table).  Per-item table scratch in units of
-// sizeof(pt): the Jacobian build keeps the affine entry of P (64 B), the Jacobian multiples 2..TS (96 B each) and the
-// suffix products of their Z's for the shared inversion (32 B each) side by side, then overwrites the front with the
-// TS affine entries the ladder reads.
+// sizeof(pt): the Jacobian build keeps the TS affine rows the ladder reads (64 B each), then the TS - 2 Z ratios of
+// the co-Z chain that built them (32 B each; the first slot holds the common denominator once the rows are scaled).
 #ifndef S256_DSM_RCB
 #define S256_DSM_JAC 1
-constexpr int DSM_TSTRIDE = (64 + (DSM_TS - 1) * 96 + (DSM_TS - 2) * 32 + 95) / 96;
+static_assert(DSM_TS >= 4, "the co-Z table needs at least two chain steps (item_dsm_table)");
+constexpr int DSM_TSTRIDE = (64 * DSM_TS + 32 * (DSM_TS - 2) + 95) / 96;
 #else
 constexpr int DSM_TSTRIDE = DSM_TS;
 #endif
@@ -387,104 +387,71 @@ S256_HD void apt_fetch64(apt &r, const apt *p) {
     r = *p;
 #endif
 }
-// Jacobian form (jac.cuh).  Table: [2..TS]P in Jacobian coordinates by doublings and mixed additions, then every row
-// is scaled to the COMMON denominator Z_all = Z_2 ... Z_TS (no inversion), which makes the TS rows affine points of
-// an isomorphic curve; every ladder addition is then a mixed one.  Layout of the item's scratch (bytes): [0, 64) P;
-// [64, 64 + 96 (TS - 1)) the Jacobian multiples 2..TS; then the suffix products Z_k ... Z_TS for k = 3..TS.  The
-// affine rows overwrite the front in ascending order: row k ends at 64 k, the first Jacobian multiple still needed
-// (k + 1) starts at 64 + 96 (k - 1).  item_dsm_table builds the multiples, item_dsm_ladder scales them and runs the
-// ladder; item_dsm is the composition.
+// Jacobian form (jac.cuh).  Table: the multiples [1..TS]P as AFFINE points of an isomorphic curve, all over the COMMON
+// denominator Z_all (no inversion), so that every ladder addition is a mixed one.  They are built as a co-Z chain
+// (Meloni's ZADDU; libsecp256k1's odd-multiples table with its "global Z" is the same construction):
+//   * DBLU from the affine key P gives 2P at Z_2 = 2y and P at that same Z;
+//   * for k = 2 .. TS - 1, ZADDU(P, kP) gives (k + 1)P and P again, both at Z_(k+1) = Z_k u_k, u_k = X(P) - X(kP).
+// No Z is ever formed: the rows are stored as they come, row k at Z_k, with the ratio u_k.  A backward pass then scales
+// row k by (r^2, r^3), r = u_k ... u_(TS-1) = Z_TS / Z_k (row TS and the last copy of P are at Z_TS already), and
+// Z_all = Z_TS = 2y r_2.  (X_k r^2, Y_k r^3) are the affine coordinates of kP on y^2 = x^3 + 7 Z_all^6; neither the
+// a = 0 doubling nor the mixed addition nor x -> beta x involves b, so the ladder runs there unchanged, and its result
+// (X', Y', Z') is (X', Y', Z' Z_all) on secp256k1.
+// No step is exceptional: u_k = 0 would mean kP = +-P, i.e. (k -+ 1)P = O with 1 <= k -+ 1 <= TS, impossible on a
+// curve of prime order; P itself is never O (every decoder substitutes G for an invalid row) and y != 0.
+// Layout of the item's scratch (bytes): [0, 64 TS) rows 1..TS; then u_2 .. u_(TS-1), 32 B each, whose first slot
+// holds Z_all once the rows are scaled.  item_dsm_table builds the rows, item_dsm_ladder runs the ladder over them;
+// item_dsm is the composition.
 // (Round 2 first divided every row by its own Z -- one safegcd inversion per item through Montgomery's trick, 20.01 ms
-// at 2^20; then one inversion per CTA, 19.14 ms, with 6 % of the warp time spent at the barrier around it; the
-// common denominator needs neither: 18.14 ms.)
+// at 2^20; then one inversion per CTA, 19.14 ms, with 6 % of the warp time spent at the barrier around it; then
+// doublings and mixed additions with prefix / suffix products of their Z's for the common denominator, 18.14 ms.)
+constexpr int DSM_U_OFF = 64 * DSM_TS;  // byte offset of the ratios (and of Z_all) in the item's scratch
 template <class F>
 S256_HD void item_dsm_table(F &f, size_t i, const apt *aff, pt *tbl) {
     char *base = reinterpret_cast<char *>(tbl + i * (size_t)DSM_TSTRIDE);
-    apt *A = reinterpret_cast<apt *>(base);
-    {
-        pt *J = reinterpret_cast<pt *>(base + 64);                          // J[k - 2] = k P
-        fe *C = reinterpret_cast<fe *>(base + 64 + 96 * (DSM_TS - 1));      // C[k - 3] = Z_k Z_(k+1) ... Z_TS
-        apt P = aff[i];
-        A[0] = P;
-        pt cur;
+    apt *A = reinterpret_cast<apt *>(base);            // A[k - 1] = row k
+    fe *U = reinterpret_cast<fe *>(base + DSM_U_OFF);  // U[k - 2] = u_k
+    apt P = aff[i];
+    apt p, q;  // P and kP at Z_k
+    jac_dblu(f, q.x, q.y, p.x, p.y, P.x, P.y);
+    A[1] = q;
 #if defined(__CUDA_ARCH__)
 #pragma unroll 1
 #endif
-        for (int k = 2; k <= DSM_TS; k += 2) {
-            pt h;
-            if (k == 2)
-                pt_from_affine(h, P);
-            else
-                h = J[k / 2 - 2];
-            jac_double(f, cur, h);
-            J[k - 2] = cur;
-            if (k < DSM_TS) {
-                jac_add_mixed_nocheck(f, cur, cur, P.x, P.y);
-                J[k - 1] = cur;
-            }
-        }
-        fe run = cur.z;  // Z_TS
-#if defined(__CUDA_ARCH__)
-#pragma unroll 1
-#endif
-        for (int k = DSM_TS - 1; k >= 2; k--) {
-            C[k + 1 - 3] = run;
-            fe zk = J[k - 2].z;
-            f.mul(run, run, zk);
-        }
+    for (int k = 2; k < DSM_TS; k++) {
+        fe u;
+        jac_zaddu(f, p.x, p.y, q.x, q.y, u);
+        A[k] = q;
+        U[k - 2] = u;
     }
+    A[0] = p;
+    fe r = U[DSM_TS - 3];
+#if defined(__CUDA_ARCH__)
+#pragma unroll 1
+#endif
+    for (int k = DSM_TS - 1; k >= 2; k--) {
+        if (k < DSM_TS - 1) {
+            fe uk = U[k - 2];
+            f.mul(r, r, uk);
+        }
+        apt a = A[k - 1];
+        fe rr;
+        f.sqr(rr, r);
+        f.mul(a.x, a.x, rr);
+        f.mul(rr, rr, r);
+        f.mul(a.y, a.y, rr);
+        A[k - 1] = a;
+    }
+    fe zall;
+    f.mul2(zall, P.y);
+    f.mul(zall, zall, r);
+    U[0] = zall;  // for the way back
 }
-// inv = (Z_2 ... Z_TS)^-1 of this item's table
 template <class F>
 S256_HD void item_dsm_ladder(F &f, size_t i, size_t n, const sc *u1s, const int8_t *dig1, const int8_t *dig2,
                              const uint8_t *sfl, pt *tbl, pt *res, const apt *comb) {
     char *base = reinterpret_cast<char *>(tbl + i * (size_t)DSM_TSTRIDE);
-    apt *A = reinterpret_cast<apt *>(base);
-    {
-        pt *J = reinterpret_cast<pt *>(base + 64);
-        fe *C = reinterpret_cast<fe *>(base + 64 + 96 * (DSM_TS - 1));
-        // No inversion at all: every row is brought to the COMMON denominator Z_all = Z_2 ... Z_TS instead of to 1.
-        // (X_k w^2, Y_k w^3) with w = Z_all / Z_k = (Z_2 .. Z_(k-1)) (Z_(k+1) .. Z_TS) are the affine coordinates of k P
-        // on the isomorphic curve y^2 = x^3 + 7 Z_all^6; neither the a = 0 doubling nor the mixed addition nor x -> beta x
-        // involves b, so the ladder runs there unchanged, and its result (X', Y', Z') is (X', Y', Z' Z_all) on secp256k1.
-        // Same 5 M + S per row as the division by Z_k, minus the inversion and the CTA-wide exchange around it.
-        fe pre = fe_one();
-#if defined(__CUDA_ARCH__)
-#pragma unroll 1
-#endif
-        for (int k = 2; k <= DSM_TS; k++) {
-            pt jk = J[k - 2];
-            fe w, w2;
-            if (k == 2) {
-                w = C[0];
-                pre = jk.z;
-            } else {
-                if (k < DSM_TS) {
-                    fe ck = C[k + 1 - 3];
-                    f.mul(w, pre, ck);
-                } else {
-                    w = pre;
-                }
-                f.mul(pre, pre, jk.z);
-            }
-            apt a;
-            f.sqr(w2, w);
-            f.mul(a.x, jk.x, w2);
-            f.mul(w2, w2, w);
-            f.mul(a.y, jk.y, w2);
-            A[k - 1] = a;
-        }
-        {
-            apt a = A[0];
-            fe zz;
-            f.sqr(zz, pre);
-            f.mul(a.x, a.x, zz);
-            f.mul(zz, zz, pre);
-            f.mul(a.y, a.y, zz);
-            A[0] = a;
-            C[0] = pre;  // Z_all, for the way back
-        }
-    }
+    const apt *A = reinterpret_cast<const apt *>(base);
     uint32_t fl = sfl[i];
     // the identity is the flag; the coordinates underneath are all zero, which every doubling maps to all zero (with
     // (0 : 1 : 0) they become small negative numbers, i.e. values next to 2^256, whose products take the folds' rare path)
@@ -534,7 +501,7 @@ S256_HD void item_dsm_ladder(F &f, size_t i, size_t n, const sc *u1s, const int8
         }
     }
     if (!inf) {  // back from the isomorphic curve before the G half, whose rows are points of secp256k1 itself
-        fe zall = reinterpret_cast<const fe *>(base + 64 + 96 * (DSM_TS - 1))[0];
+        fe zall = reinterpret_cast<const fe *>(base + DSM_U_OFF)[0];
         f.mul(acc.z, acc.z, zall);
     }
     sc u1 = u1s[i];
