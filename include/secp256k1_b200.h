@@ -188,6 +188,20 @@ int s256_schnorr_verify(s256_ctx *ctx, const uint8_t *pkx32, const uint8_t *msg,
 int s256_schnorr_verify_dev(s256_ctx *ctx, const uint8_t *d_pkx32, const uint8_t *d_msg, size_t msg_len,
                             const uint8_t *d_sig64, size_t n, uint8_t *d_ok, void *stream);
 
+/* BIP-340 batch verification (BIP-340 "Batch Verification"; per item: bitcoin.SchnorrPublicKey.Verify,
+ * secec/bitcoin/schnorr.go:221, incl. lift_x :257).  Inputs are laid out as for s256_schnorr_verify.
+ * *ok = 1 iff every row would verify; 0 otherwise (except with probability <= 2^-127 per call when
+ * some row is invalid).  n == 0 gives 1.  Variable time (public data).
+ * One equation, (sum a_i s_i) G = sum a_i R_i + sum (a_i e_i) P_i with R_i = lift_x(r_i), a_0 = 1 and 128-bit a_i
+ * derived from a hash tree over all the rows (DESIGN.md), checked by one multi-scalar multiplication.  A row is
+ * rejected, and with it the batch, when its key does not lift_x, r >= p, r is not the x-coordinate of a curve point, or
+ * s >= n.  To find the invalid rows of a rejected batch, run s256_schnorr_verify on it.  The _dev form writes the
+ * verdict byte to device memory and does not synchronise.  S256_ERR_ARG for a context with max_batch < 2. */
+int s256_schnorr_batch_verify(s256_ctx *ctx, const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
+                              const uint8_t *sig64, size_t n, uint8_t *ok);
+int s256_schnorr_batch_verify_dev(s256_ctx *ctx, const uint8_t *d_pkx32, const uint8_t *d_msg, size_t msg_len,
+                                  const uint8_t *d_sig64, size_t n, uint8_t *d_ok, void *stream);
+
 /* --- bitcoin.SchnorrPrivateKey.Sign (secec/bitcoin/schnorr.go:111-147 -> signSchnorr :322): BIP-340
  *     signing with caller-supplied auxiliary randomness (32 B per row; the reference draws it from
  *     its entropy source, :130-141).  priv32 as for NewPrivateKey; constant time. */

@@ -39,6 +39,7 @@ EXPORTED_SYMBOLS = [
     "s256_ecdsa_recover", "s256_ecdsa_recover_dev",
     "s256_ecdsa_sign_rfc6979", "s256_ecdsa_sign_rfc6979_dev",
     "s256_schnorr_verify", "s256_schnorr_verify_dev", "s256_schnorr_sign", "s256_schnorr_sign_dev",
+    "s256_schnorr_batch_verify", "s256_schnorr_batch_verify_dev",
     "s256_msm", "s256_msm_partial", "s256_msm_combine", "s256_msm_dev", "s256_msm_sharded", "s256_msm_sharded_dev",
     "s256_comm_unique_id", "s256_comm_init", "s256_comm_free", "s256_msm_plan", "s256_hash_to_curve", "s256_expand_message_xmd",
     "s256_debug_ladder_add_count", "s256_mac32_k_dsm",
@@ -516,6 +517,33 @@ class Engine:
         self._check(self._lib.s256_schnorr_verify(self._ctx, self._hp(pk), self._hp(m), C.c_size_t(m.shape[1] if n else 0),
                                                   self._hp(sg), C.c_size_t(n), self._hp(ok)), "schnorr_verify")
         return ok
+
+    # -- BIP-340 batch verification: one verdict for the whole batch ----------------------------
+    def schnorr_batch_verify(self, pkx32, msg, sig64):
+        """True iff every row would pass schnorr_verify (one randomized multi-scalar multiplication; a batch with an
+        invalid row is accepted with probability <= 2^-127).  With CUDA tensors: a (1,) uint8 tensor, not synchronised."""
+        if _is_torch_cuda(pkx32):
+            import torch
+            n = pkx32.numel() // 32
+            msg_len = msg.numel() // n if n else 0
+            if sig64.numel() != 64 * n or msg.numel() != msg_len * n:
+                raise ValueError("length mismatch")
+            ok = torch.empty(1, dtype=torch.uint8, device=pkx32.device)
+            a = self._dev_args(pkx32, msg, sig64, ok)
+            self._check(self._lib.s256_schnorr_batch_verify_dev(self._ctx, a[0], a[1], C.c_size_t(msg_len), a[2], C.c_size_t(n),
+                                                                a[3], self._stream()), "schnorr_batch_verify_dev")
+            return ok
+        pk, sg = _host(pkx32, 32), _host(sig64, 64)
+        n = len(pk)
+        m = _host(msg, 0)
+        msg_len = m.size // n if n else 0
+        if len(sg) != n or m.size != msg_len * n:
+            raise ValueError("length mismatch")
+        m = m.reshape(n, msg_len)
+        ok = C.c_uint8(0)
+        self._check(self._lib.s256_schnorr_batch_verify(self._ctx, self._hp(pk), self._hp(m), C.c_size_t(msg_len), self._hp(sg),
+                                                        C.c_size_t(n), C.byref(ok)), "schnorr_batch_verify")
+        return bool(ok.value)
 
     # -- bitcoin.SchnorrPrivateKey.Sign (secec/bitcoin/schnorr.go:111,322) ---------------------
     def schnorr_sign(self, priv32, msg, aux32):

@@ -10,7 +10,7 @@ LIBDIR = os.path.join(HERE, "lib")
 # S256_LIB=<path> selects a prebuilt variant (tuning experiments); it is never rebuilt.
 LIB = os.environ.get("S256_LIB") or os.path.join(LIBDIR, "libsecp256k1_b200.so")
 SOURCES = ["api.cu", "api_msm.cu", "api_sign.cu", "api_h2c.cu", "kern_ct.cu", "codecs.cpp"]
-HEADERS = ["fe.cuh", "sc.cuh", "point.cuh", "sha256.cuh", "kernels.cuh", "microbench.cuh", "launchers.h", "msm.cuh", "fe_sqr_gen.cuh", "ctx.h", "h2c.cuh", "fe_vt.cuh", "coop.cuh", "modinv.cuh", "fe_mul_gen.cuh", "jac.cuh"]
+HEADERS = ["fe.cuh", "sc.cuh", "point.cuh", "sha256.cuh", "kernels.cuh", "microbench.cuh", "launchers.h", "msm.cuh", "fe_sqr_gen.cuh", "ctx.h", "h2c.cuh", "fe_vt.cuh", "coop.cuh", "modinv.cuh", "fe_mul_gen.cuh", "jac.cuh", "batch.cuh"]
 
 
 def nvcc_cmd(extra=(), out=None):

@@ -422,7 +422,8 @@ extern "C" void s256_free(s256_ctx *ctx) {
                         ctx->cstat, ctx->tbl,   ctx->res, ctx->in_a, ctx->in_b, ctx->in_c, ctx->out, ctx->st,
                         ctx->sink, ctx->msm_counts, ctx->msm_offsets, ctx->msm_cursor, ctx->msm_entries, ctx->msm_flag,
                         ctx->msm_buckets, ctx->msm_win, ctx->msm_acc, ctx->msm_tmp, ctx->msm_cub, ctx->msm_nsl, ctx->msm_sloff,
-                        ctx->msm_perm, ctx->msm_hist, ctx->msm_range, ctx->msm_part, ctx->msm_sbkt, ctx->comm_buf, ctx->msm_aff2, ctx->msm_half, ctx->msm_bsum};
+                        ctx->msm_perm, ctx->msm_hist, ctx->msm_range, ctx->msm_part, ctx->msm_sbkt, ctx->comm_buf, ctx->msm_aff2, ctx->msm_half, ctx->msm_bsum,
+                        ctx->bat};
         for (void *p : ptrs)
             if (p) cudaFree(p);
         if (ctx->stream) cudaStreamDestroy(ctx->stream);

@@ -1,6 +1,8 @@
-// api_msm.cu -- Point.MultiScalarMult[Vartime]: the Pippenger kernels (msm.cuh) and their entry points.
+// api_msm.cu -- Point.MultiScalarMult[Vartime]: the Pippenger kernels (msm.cuh) and their entry points, and the
+// BIP-340 batch verification built on them (batch.cuh).
 #include "ctx.h"
 #include "msm.cuh"
+#include "batch.cuh"
 #include "coop.cuh"
 #include <cub/device/device_scan.cuh>
 #include <dlfcn.h>
@@ -331,11 +333,8 @@ static int msm_ensure(s256_ctx *ctx) {
     return S256_SUCCESS;
 }
 
-// one chunk (device pointers): msm_acc (+)= sum k_i P_i
-static int chunk_msm(s256_ctx *ctx, const uint8_t *k32, const uint8_t *pt65, size_t n, int vartime, int first,
-                     cudaStream_t s) {
-    s256_launch_decode_uncompressed(ctx, pt65, n, ctx->aff, ctx->pvalid, s);
-    LAUNCH(ctx, k_any_invalid, grid_for(n), 0, s, ctx->pvalid, n, ctx->msm_flag);
+// one chunk of points already in ctx->aff (device pointers): msm_acc (+)= sum k_i P_i
+static int chunk_msm_body(s256_ctx *ctx, const uint8_t *k32, size_t n, int vartime, int first, cudaStream_t s) {
     if (!vartime || n < 32) {
         // constant-time flavour (and tiny inputs): ct ladder per item, then a sum tree
         s256_launch_scalar_mult_ct(n, ctx->aff, k32, ctx->tbl, ctx->res, s);
@@ -399,6 +398,13 @@ static int chunk_msm(s256_ctx *ctx, const uint8_t *k32, const uint8_t *pt65, siz
     k_msm_final<<<1, 32, 0, s>>>(pl, ctx->msm_win, ctx->msm_acc, first);
     ctx->launches.fetch_add(5, std::memory_order_relaxed);
     return S256_SUCCESS;
+}
+// one chunk of encoded points: decode into ctx->aff (a failed decode sets msm_flag), then the sum
+static int chunk_msm(s256_ctx *ctx, const uint8_t *k32, const uint8_t *pt65, size_t n, int vartime, int first,
+                     cudaStream_t s) {
+    s256_launch_decode_uncompressed(ctx, pt65, n, ctx->aff, ctx->pvalid, s);
+    LAUNCH(ctx, k_any_invalid, grid_for(n), 0, s, ctx->pvalid, n, ctx->msm_flag);
+    return chunk_msm_body(ctx, k32, n, vartime, first, s);
 }
 
 // host pointers -> msm_acc holds the projective sum; *invalid = 1 if a point failed to decode
@@ -492,6 +498,253 @@ extern "C" int s256_msm_combine(s256_ctx *ctx, const uint8_t *partials96, size_t
         return S256_SUCCESS;
     }
     return msm_finish(ctx, out65, status);
+}
+
+
+// ---------------------------------------------------------------------------
+// BIP-340 batch verification (batch.cuh): one verdict for a whole batch of Schnorr signatures, from one randomized
+// multi-scalar multiplication.
+//
+// Rows go in chunks of C = the largest power of two <= cap / 2, so that a chunk's 2C MSM points fit the per-chunk
+// scratch and the chunk roots are nodes of the batch's hash tree.  Pass 1 hashes the rows into leaves (ctx->u1) and
+// folds each chunk to its root (k_batch_tree); k_batch_seed folds the roots into the seed.  Pass 2 turns each chunk into
+// the 2c MSM rows (-R_i, a_i), (-P_i, a_i e_i) in ctx->aff / ctx->out plus per-CTA sums of a_i s_i (ctx->u1, folded into
+// one scalar by k_batch_fold) and runs them through the Pippenger body.  The finish adds (sum a_i s_i) G and tests the
+// sum for the identity.
+// ---------------------------------------------------------------------------
+constexpr int BATCH_SEG = 2 * S256_TPB;  // nodes one CTA of k_batch_tree folds into one
+// ctx->bat, in 32-bit words: the seed, the scalar sum (limbs), the scalar sum (big-endian bytes), one root per chunk
+constexpr size_t BAT_SEED = 0, BAT_SUM = 8, BAT_SUM_BE = 16, BAT_ROOTS = 24;
+
+__global__ void __launch_bounds__(S256_TPB) k_batch_leaves(const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
+                                                           const uint8_t *sig64, size_t n, uint32_t *leaves) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint32_t h[8];
+    batch_leaf(h, pkx32 + 32 * i, sig64 + 64 * i, msg + msg_len * i, msg_len);
+    uint4 *o = reinterpret_cast<uint4 *>(leaves + 8 * i);
+    o[0] = make_uint4(h[0], h[1], h[2], h[3]);
+    o[1] = make_uint4(h[4], h[5], h[6], h[7]);
+}
+// out[b] = the node over in[b * BATCH_SEG, ...) by the tree rule: the first level from global memory, the rest in
+// shared memory.  Segments start at multiples of 2^8, so out[] is a level of the whole tree.
+__global__ void __launch_bounds__(S256_TPB) k_batch_tree(const uint32_t *in, size_t m, uint32_t *out) {
+    __shared__ uint32_t sh[S256_TPB][8];
+    const size_t base = (size_t)blockIdx.x * BATCH_SEG;
+    const uint32_t t = threadIdx.x;
+    uint32_t cnt = (uint32_t)(m - base < (size_t)BATCH_SEG ? m - base : (size_t)BATCH_SEG);
+    uint32_t h[8] = {};
+    if (2 * t + 1 < cnt) {
+        batch_node(h, in + 8 * (base + 2 * t), in + 8 * (base + 2 * t + 1));
+    } else if (2 * t < cnt) {
+        for (int k = 0; k < 8; k++) h[k] = in[8 * (base + 2 * t) + k];
+    }
+    for (int k = 0; k < 8; k++) sh[t][k] = h[k];
+    cnt = (cnt + 1) / 2;
+    __syncthreads();
+    while (cnt > 1) {
+        uint32_t up = (cnt + 1) / 2;
+        if (t < up) {
+            if (2 * t + 1 < cnt) {
+                batch_node(h, sh[2 * t], sh[2 * t + 1]);
+            } else {
+                for (int k = 0; k < 8; k++) h[k] = sh[2 * t][k];
+            }
+        }
+        __syncthreads();
+        if (t < up)
+            for (int k = 0; k < 8; k++) sh[t][k] = h[k];
+        __syncthreads();
+        cnt = up;
+    }
+    if (t < 8) out[8 * (size_t)blockIdx.x + t] = sh[0][t];
+}
+// chunk roots -> seed (one thread; a batch has few chunks)
+__global__ void k_batch_seed(uint32_t *bat, size_t chunks, uint64_t n) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    batch_tree_fold(bat + BAT_ROOTS, chunks);
+    batch_seed(bat + BAT_SEED, bat + BAT_ROOTS, n);
+}
+// rows [off, off + n) of the batch -> MSM rows 2i, 2i + 1 of the chunk, part[CTA] = the CTA's sum of a_i s_i,
+// flag |= a rejected row
+__global__ void __launch_bounds__(S256_TPB) k_batch_prepare(const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
+                                                            const uint8_t *sig64, size_t n, size_t off, const uint32_t *seed_in,
+                                                            apt *aff2, uint8_t *k2, sc *part, uint32_t *flag) {
+    __shared__ sc sh[S256_TPB];
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int t = threadIdx.x;
+    sc as = sc_zero();
+    if (i < n) {
+        uint32_t seed[8];
+        for (int k = 0; k < 8; k++) seed[k] = seed_in[k];
+        uint32_t ok = item_batch_prepare(aff2 + 2 * i, k2 + 64 * i, as, pkx32 + 32 * i, msg + msg_len * i, msg_len,
+                                         sig64 + 64 * i, seed, (uint64_t)(off + i));
+        if (!ok) atomicOr(flag, 1u);
+    }
+    sh[t] = as;
+    __syncthreads();
+    for (int stride = S256_TPB / 2; stride >= 1; stride >>= 1) {
+        if (t < stride) {
+            sc a = sh[t], b = sh[t + stride];
+            sc_add(a, a, b);
+            sh[t] = a;
+        }
+        __syncthreads();
+    }
+    if (t == 0) part[blockIdx.x] = sh[0];
+}
+// the scalar sum (+)= the m CTA sums (first = overwrite), kept as limbs and as big-endian bytes.  One CTA.
+__global__ void __launch_bounds__(S256_TPB) k_batch_fold(const sc *part, size_t m, uint32_t *bat, int first) {
+    __shared__ sc sh[S256_TPB];
+    const int t = threadIdx.x;
+    sc acc = sc_zero();
+    for (size_t j = t; j < m; j += S256_TPB) {
+        sc q = part[j];
+        sc_add(acc, acc, q);
+    }
+    sh[t] = acc;
+    __syncthreads();
+    for (int stride = S256_TPB / 2; stride >= 1; stride >>= 1) {
+        if (t < stride) {
+            sc a = sh[t], b = sh[t + stride];
+            sc_add(a, a, b);
+            sh[t] = a;
+        }
+        __syncthreads();
+    }
+    if (t == 0) {
+        sc r = sh[0];
+        sc *sum = reinterpret_cast<sc *>(bat + BAT_SUM);
+        if (!first) {
+            sc a = *sum;
+            sc_add(r, r, a);
+        }
+        *sum = r;
+        sc_to_be32(reinterpret_cast<uint8_t *>(bat + BAT_SUM_BE), r);
+    }
+}
+// ok = no row was rejected and the sum is the identity
+__global__ void k_batch_verdict(const uint32_t *flag, const pt *acc, uint8_t *ok) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    pt a = *acc;
+    *ok = (uint8_t)((uint32_t)(*flag == 0) & fe_is_zero(a.z));
+}
+
+static size_t batch_chunk(const s256_ctx *ctx) {  // the largest power of two <= cap / 2
+    size_t c = 1;
+    while (4 * c <= ctx->cap) c *= 2;
+    return c;
+}
+static int batch_ensure(s256_ctx *ctx, size_t chunks) {
+    if (chunks <= ctx->bat_chunks) return S256_SUCCESS;
+    if (chunks < 16) chunks = 16;
+    uint32_t *fresh = nullptr;
+    CK(cudaMalloc(&fresh, (BAT_ROOTS + 8 * chunks) * 4));
+    if (ctx->bat) cudaFree(ctx->bat);  // synchronises the device: no call still reads the old array
+    ctx->bat = fresh;
+    ctx->bat_chunks = chunks;
+    return S256_SUCCESS;
+}
+struct batch_rows {
+    const uint8_t *pkx, *msg, *sig;
+};
+// n >= 1 rows; rows(off, c, pass, r) gives the device rows of a chunk (the host form copies them in first).
+// The verdict byte goes to d_ok; nothing is synchronised.
+template <typename F>
+static int batch_verify_run(s256_ctx *ctx, size_t n, size_t msg_len, F rows, uint8_t *d_ok, cudaStream_t s) {
+    int rc = msm_ensure(ctx);
+    if (rc != S256_SUCCESS) return rc;
+    const size_t C = batch_chunk(ctx), chunks = (n + C - 1) / C;
+    rc = batch_ensure(ctx, chunks);
+    if (rc != S256_SUCCESS) return rc;
+    uint32_t *leaves = reinterpret_cast<uint32_t *>(ctx->u1);
+    uint32_t *level[2] = {reinterpret_cast<uint32_t *>(ctx->res),
+                          reinterpret_cast<uint32_t *>(ctx->res) + 8 * ((C + BATCH_SEG - 1) / BATCH_SEG)};
+    batch_rows r;
+    // pass 1: leaves -> chunk roots -> seed
+    for (size_t k = 0; k < chunks; k++) {
+        const size_t off = k * C, c = n - off < C ? n - off : C;
+        rc = rows(off, c, 0, r);
+        if (rc != S256_SUCCESS) return rc;
+        LAUNCH(ctx, k_batch_leaves, grid_for(c), 0, s, r.pkx, r.msg, msg_len, r.sig, c, leaves);
+        const uint32_t *src = leaves;
+        size_t m = c;
+        int side = 0;
+        do {
+            size_t g = (m + BATCH_SEG - 1) / BATCH_SEG;
+            uint32_t *dst = g == 1 ? ctx->bat + BAT_ROOTS + 8 * k : level[side];
+            LAUNCH(ctx, k_batch_tree, (unsigned)g, 0, s, src, m, dst);
+            src = dst;
+            side ^= 1;
+            m = g;
+        } while (m > 1);
+    }
+    k_batch_seed<<<1, 1, 0, s>>>(ctx->bat, chunks, (uint64_t)n);
+    ctx->launches.fetch_add(1, std::memory_order_relaxed);
+    // pass 2: per chunk, the MSM rows and the scalar sum, then the Pippenger body
+    CK(cudaMemsetAsync(ctx->msm_flag, 0, 4, s));
+    for (size_t k = 0; k < chunks; k++) {
+        const size_t off = k * C, c = n - off < C ? n - off : C;
+        rc = rows(off, c, 1, r);
+        if (rc != S256_SUCCESS) return rc;
+        LAUNCH(ctx, k_batch_prepare, grid_for(c), 0, s, r.pkx, r.msg, msg_len, r.sig, c, off, ctx->bat + BAT_SEED, ctx->aff,
+               ctx->out, ctx->u1, ctx->msm_flag);
+        k_batch_fold<<<1, S256_TPB, 0, s>>>(ctx->u1, (size_t)grid_for(c), ctx->bat, k == 0);
+        ctx->launches.fetch_add(1, std::memory_order_relaxed);
+        rc = chunk_msm_body(ctx, ctx->out, 2 * c, 1, k == 0, s);
+        if (rc != S256_SUCCESS) return rc;
+    }
+    // finish: + (sum a_i s_i) G, then the verdict
+    s256_launch_base_mult_ct(reinterpret_cast<const uint8_t *>(ctx->bat + BAT_SUM_BE), 1, ctx->ct_tab, ctx->ct_tab_small,
+                             ctx->ct_tab_huge, ctx->res, s);
+    k_acc_point<<<1, 1, 0, s>>>(ctx->res, ctx->msm_acc, 0);
+    k_batch_verdict<<<1, 1, 0, s>>>(ctx->msm_flag, ctx->msm_acc, d_ok);
+    ctx->launches.fetch_add(3, std::memory_order_relaxed);
+    return check_launch(ctx);
+}
+extern "C" int s256_schnorr_batch_verify_dev(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
+                                             const uint8_t *sig, size_t n, uint8_t *ok, void *stream) {
+    ENTER(ctx);
+    if (!ok || (n && (!pkx || (!msg && msg_len) || !sig))) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;  // a chunk needs two MSM rows per signature
+    cudaStream_t s = (cudaStream_t)stream;
+    scratch_guard sg_(ctx, s, false);
+    if (n == 0) {
+        CK(cudaMemsetAsync(ok, 1, 1, s));
+        return S256_SUCCESS;
+    }
+    return batch_verify_run(ctx, n, msg_len, [&](size_t off, size_t, int, batch_rows &r) {
+        r = batch_rows{pkx + 32 * off, msg_len ? msg + msg_len * off : msg, sig + 64 * off};
+        return S256_SUCCESS;
+    }, ok, s);
+}
+extern "C" int s256_schnorr_batch_verify(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
+                                         const uint8_t *sig, size_t n, uint8_t *ok) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    if (!ok || (n && (!pkx || (!msg && msg_len) || !sig))) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    if (n == 0) {
+        *ok = 1;
+        return S256_SUCCESS;
+    }
+    const size_t C = batch_chunk(ctx);
+    if (int grc = grow_in_b(ctx, (msg_len ? msg_len : 1) * C)) return grc;
+    cudaStream_t s = ctx->stream;
+    const bool resident = n <= C;  // one chunk: copied once, read by both passes
+    int rc = batch_verify_run(ctx, n, msg_len, [&](size_t off, size_t c, int pass, batch_rows &r) {
+        if (pass == 0 || !resident) {
+            CK(cudaMemcpyAsync(ctx->in_a, pkx + 32 * off, 32 * c, cudaMemcpyHostToDevice, s));
+            if (msg_len) CK(cudaMemcpyAsync(ctx->in_b, msg + msg_len * off, msg_len * c, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(ctx->in_c, sig + 64 * off, 64 * c, cudaMemcpyHostToDevice, s));
+        }
+        r = batch_rows{ctx->in_a, ctx->in_b, ctx->in_c};
+        return S256_SUCCESS;
+    }, ctx->st, s);
+    if (rc != S256_SUCCESS) return rc;
+    CK(cudaMemcpyAsync(ok, ctx->st, 1, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));  // the one host synchronisation of the call
+    return check_launch(ctx);
 }
 
 

@@ -55,6 +55,9 @@ struct s256_ctx {
     void *msm_half = nullptr; // the 2n 128-bit scalar halves
     void *msm_cub = nullptr;
     size_t msm_cub_bytes = 0;
+    // BIP-340 batch verification (api_msm.cu): seed, the scalar sum and its bytes, then one root per chunk
+    uint32_t *bat = nullptr;
+    size_t bat_chunks = 0;
     // optional per-kernel timing of the dominant kernel (bench.py roofline)
     bool profiling = false;
     // sub-chunks per host-pointer call (S256_PIPE_PARTS).  Measured (scripts/e2e_parts.py): splitting does not

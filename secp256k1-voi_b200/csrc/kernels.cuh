@@ -314,6 +314,21 @@ S256_HD void group_recover_scalars(size_t t, size_t stride, size_t n, const uint
     }
 }
 
+// e = H_challenge(r || P || m) mod n (secec/bitcoin/schnorr.go:445-446) for one row: sg = r || s, pkx = x(P)
+S256_HD void item_schnorr_challenge(sc &e, const uint8_t *sg, const uint8_t *pkx, const uint8_t *m, size_t msg_len) {
+    uint8_t eb[32];
+    if (msg_len == 32) {  // fixed layout: the tag midstate plus two compressions, all in words
+        uint32_t rw[8], pw[8], mw[8], ew[8];
+        be32_words(rw, sg);
+        be32_words(pw, pkx);
+        be32_words(mw, m);
+        bip340_tagged_96(ew, TAG_CHALLENGE, rw, pw, mw);
+        words_be32(eb, ew);
+    } else {
+        bip340_challenge(eb, sg, pkx, m, msg_len);
+    }
+    sc_from_be32(e, eb);
+}
 // secec/bitcoin/schnorr.go:420-449: r < p, s < n (zero allowed),
 // e = H(r||P||m) mod n; R = s*G + (-e)*P (:244-245)
 S256_HD void item_schnorr_scalars(size_t i, size_t n, const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
@@ -323,18 +338,7 @@ S256_HD void item_schnorr_scalars(size_t i, size_t n, const uint8_t *pkx32, cons
     fe_from_be32(r, sg);
     sc s, e, ne;
     uint32_t ok = fe_limbs_are_canonical(r) & (1u - sc_from_be32(s, sg + 32));
-    uint8_t eb[32];
-    if (msg_len == 32) {  // fixed layout: the tag midstate plus two compressions, all in words
-        uint32_t rw[8], pw[8], mw[8], ew[8];
-        be32_words(rw, sg);
-        be32_words(pw, pkx32 + 32 * i);
-        be32_words(mw, msg + 32 * i);
-        bip340_tagged_96(ew, TAG_CHALLENGE, rw, pw, mw);
-        words_be32(eb, ew);
-    } else {
-        bip340_challenge(eb, sg, pkx32 + 32 * i, msg + msg_len * i, msg_len);
-    }
-    sc_from_be32(e, eb);
+    item_schnorr_challenge(e, sg, pkx32 + 32 * i, msg + msg_len * i, msg_len);
     sc_neg(ne, e);
     item_store_scalars(s, ne, ok, i, n, u1_out, dig1, dig2, sfl);
 }

@@ -119,6 +119,21 @@ func (e *Engine) SchnorrVerifyBatch(pkx32, msgs []byte, msgLen int, sig64 []byte
 	return out, nil
 }
 
+// SchnorrBatchVerify is BIP-340 batch verification: true iff every row would pass bitcoin.SchnorrPublicKey.Verify
+// (one randomized multi-scalar multiplication; a batch with an invalid row passes with probability <= 2^-127).
+// SchnorrVerifyBatch finds the bad rows of a rejected batch.
+func (e *Engine) SchnorrBatchVerify(pkx32, msgs []byte, msgLen int, sig64 []byte) (bool, error) {
+	n := len(pkx32) / 32
+	if len(pkx32) != 32*n || len(msgs) != msgLen*n || len(sig64) != 64*n {
+		panic("secp256k1b200: SchnorrBatchVerify: length mismatch")
+	}
+	var ok C.uint8_t
+	if err := e.err(C.s256_schnorr_batch_verify(e.ctx, ptr(pkx32), ptr(msgs), C.size_t(msgLen), ptr(sig64), C.size_t(n), &ok)); err != nil {
+		return false, err
+	}
+	return ok == 1, nil
+}
+
 // ScalarBaseMultBatch is Point.ScalarBaseMult + UncompressedBytes (constant time).
 func (e *Engine) ScalarBaseMultBatch(scalars []*secp256k1.Scalar) ([]*secp256k1.Point, error) {
 	n := len(scalars)

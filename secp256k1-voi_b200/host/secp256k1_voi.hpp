@@ -846,6 +846,14 @@ inline void SchnorrVerifyBatch(const uint8_t *pkx32, const uint8_t *msg, size_t 
                                uint8_t *ok, Engine &e = Engine::Default()) {
     e.check(s256_schnorr_verify(e.ctx(), pkx32, msg, msg_len, sig64, n, ok), "SchnorrVerifyBatch");
 }
+// BIP-340 batch verification: true iff every row would pass SchnorrPublicKey.Verify (one randomized multi-scalar
+// multiplication; a batch with an invalid row passes with probability <= 2^-127).  SchnorrVerifyBatch finds the bad rows.
+inline bool SchnorrBatchVerify(const uint8_t *pkx32, const uint8_t *msg, size_t msg_len, const uint8_t *sig64, size_t n,
+                               Engine &e = Engine::Default()) {
+    uint8_t ok = 0;
+    e.check(s256_schnorr_batch_verify(e.ctx(), pkx32, msg, msg_len, sig64, n, &ok), "SchnorrBatchVerify");
+    return ok == 1;
+}
 }  // namespace bitcoin
 
 namespace h2c {
