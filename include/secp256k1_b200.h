@@ -296,6 +296,13 @@ double s256_mac32_per_item(const char *entry_point);
  * those counts per item. */
 int s256_debug_ladder_add_count(s256_ctx *ctx, size_t n, uint64_t *adds_first_half, uint64_t *adds_lambda_half);
 double s256_mac32_k_dsm(double adds_per_item, double beta_muls_per_item);
+/* The equation s256_schnorr_batch_verify checks for the same host rows, as its kernels build it (for tests): the
+ * 32-byte seed; per row the two MSM scalars a_i and a_i e_i mod n (k64: 2 x 32 B big-endian) and the two points -R_i
+ * and -P_i (pts128: 2 x X||Y, 32 B big-endian each; G with scalar 0 for a rejected row); sum32 = sum a_i s_i mod n
+ * big-endian; *rejected = 1 if some row was rejected.  Chunks as in the verification.  n >= 1. */
+int s256_debug_schnorr_batch_rows(s256_ctx *ctx, const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
+                                  const uint8_t *sig64, size_t n, uint8_t *seed32, uint8_t *k64, uint8_t *pts128,
+                                  uint8_t *sum32, uint8_t *rejected);
 
 #if defined(__GNUC__)
 #pragma GCC visibility pop

@@ -43,7 +43,7 @@ EXPORTED_SYMBOLS = [
     "s256_msm", "s256_msm_partial", "s256_msm_combine", "s256_msm_dev", "s256_msm_sharded", "s256_msm_sharded_dev",
     "s256_comm_unique_id", "s256_comm_init", "s256_comm_free", "s256_msm_plan", "s256_hash_to_curve", "s256_expand_message_xmd",
     "s256_debug_ladder_add_count", "s256_mac32_k_dsm",
-    "s256_debug_gen_table", "s256_debug_field_op", "s256_microbench_imad",
+    "s256_debug_gen_table", "s256_debug_field_op", "s256_debug_schnorr_batch_rows", "s256_microbench_imad",
     "s256_microbench_variant", "s256_microbench_fe_mul", "s256_profile_enable", "s256_profile_read",
     "s256_launch_count", "s256_mac32_per_item", "s256_host_alloc", "s256_host_free",
 ]
@@ -699,6 +699,24 @@ class Engine:
         self._check(self._lib.s256_debug_field_op(self._ctx, int(op), self._hp(a), self._hp(b), C.c_size_t(len(a)),
                                                   self._hp(out)), "debug_field_op")
         return out
+
+    def debug_schnorr_batch_rows(self, pkx32, msg, sig64):
+        """What schnorr_batch_verify checks for these host rows: (seed (32,), k (n, 2, 32) = a_i and a_i e_i mod n,
+        pts (n, 2, 64) = -R_i and -P_i as X||Y (G for a rejected row), sum (32,) = sum a_i s_i mod n, rejected),
+        all big-endian bytes."""
+        pk, sg = _host(pkx32, 32), _host(sig64, 64)
+        n = len(pk)
+        m = _host(msg, 0)
+        msg_len = m.size // n if n else 0
+        if n == 0 or len(sg) != n or m.size != msg_len * n:
+            raise ValueError("length mismatch or empty batch")
+        seed, k, pts, ssum, rej = (np.zeros(32, np.uint8), np.zeros((n, 2, 32), np.uint8), np.zeros((n, 2, 64), np.uint8),
+                                   np.zeros(32, np.uint8), C.c_uint8(0))
+        self._check(self._lib.s256_debug_schnorr_batch_rows(self._ctx, self._hp(pk), self._hp(m), C.c_size_t(msg_len),
+                                                            self._hp(sg), C.c_size_t(n), self._hp(seed), self._hp(k),
+                                                            self._hp(pts), self._hp(ssum), C.byref(rej)),
+                    "debug_schnorr_batch_rows")
+        return seed.tobytes(), k, pts, ssum.tobytes(), bool(rej.value)
 
     def profile_enable(self, on=True):
         self._check(self._lib.s256_profile_enable(self._ctx, int(bool(on))), "profile_enable")

@@ -6,6 +6,7 @@
 #include "coop.cuh"
 #include <cub/device/device_scan.cuh>
 #include <dlfcn.h>
+#include <functional>
 #include <nccl.h>  // types only: the library is resolved at run time (no link-time dependency on NCCL)
 
 // ---- Pippenger MSM (msm.cuh) -------------------------------------------------
@@ -648,10 +649,13 @@ static int batch_ensure(s256_ctx *ctx, size_t chunks) {
 struct batch_rows {
     const uint8_t *pkx, *msg, *sig;
 };
+// chunk_done(off, c): called once per chunk while its MSM rows are in ctx->out / ctx->aff (s256_debug_schnorr_batch_rows)
+using batch_chunk_fn = std::function<int(size_t, size_t)>;
 // n >= 1 rows; rows(off, c, pass, r) gives the device rows of a chunk (the host form copies them in first).
-// The verdict byte goes to d_ok; nothing is synchronised.
+// The verdict byte goes to d_ok; nothing is synchronised unless chunk_done does.
 template <typename F>
-static int batch_verify_run(s256_ctx *ctx, size_t n, size_t msg_len, F rows, uint8_t *d_ok, cudaStream_t s) {
+static int batch_verify_run(s256_ctx *ctx, size_t n, size_t msg_len, F rows, uint8_t *d_ok, cudaStream_t s,
+                            const batch_chunk_fn &chunk_done = nullptr) {
     int rc = msm_ensure(ctx);
     if (rc != S256_SUCCESS) return rc;
     const size_t C = batch_chunk(ctx), chunks = (n + C - 1) / C;
@@ -691,6 +695,7 @@ static int batch_verify_run(s256_ctx *ctx, size_t n, size_t msg_len, F rows, uin
                ctx->out, ctx->u1, ctx->msm_flag);
         k_batch_fold<<<1, S256_TPB, 0, s>>>(ctx->u1, (size_t)grid_for(c), ctx->bat, k == 0);
         ctx->launches.fetch_add(1, std::memory_order_relaxed);
+        if (chunk_done && (rc = chunk_done(off, c)) != S256_SUCCESS) return rc;
         rc = chunk_msm_body(ctx, ctx->out, 2 * c, 1, k == 0, s);
         if (rc != S256_SUCCESS) return rc;
     }
@@ -718,6 +723,24 @@ extern "C" int s256_schnorr_batch_verify_dev(s256_ctx *ctx, const uint8_t *pkx, 
         return S256_SUCCESS;
     }, ok, s);
 }
+// The host form's rows: a batch of one chunk is copied in once and read by both passes, a longer one chunk by chunk in
+// each pass.  The verdict byte goes to ctx->st.
+static int batch_verify_host(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len, const uint8_t *sig,
+                             size_t n, const batch_chunk_fn &chunk_done = nullptr) {
+    const size_t C = batch_chunk(ctx);
+    if (int grc = grow_in_b(ctx, (msg_len ? msg_len : 1) * C)) return grc;
+    cudaStream_t s = ctx->stream;
+    const bool resident = n <= C;
+    return batch_verify_run(ctx, n, msg_len, [&](size_t off, size_t c, int pass, batch_rows &r) {
+        if (pass == 0 || !resident) {
+            CK(cudaMemcpyAsync(ctx->in_a, pkx + 32 * off, 32 * c, cudaMemcpyHostToDevice, s));
+            if (msg_len) CK(cudaMemcpyAsync(ctx->in_b, msg + msg_len * off, msg_len * c, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(ctx->in_c, sig + 64 * off, 64 * c, cudaMemcpyHostToDevice, s));
+        }
+        r = batch_rows{ctx->in_a, ctx->in_b, ctx->in_c};
+        return S256_SUCCESS;
+    }, ctx->st, s, chunk_done);
+}
 extern "C" int s256_schnorr_batch_verify(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
                                          const uint8_t *sig, size_t n, uint8_t *ok) {
     ENTER(ctx);
@@ -728,22 +751,43 @@ extern "C" int s256_schnorr_batch_verify(s256_ctx *ctx, const uint8_t *pkx, cons
         *ok = 1;
         return S256_SUCCESS;
     }
-    const size_t C = batch_chunk(ctx);
-    if (int grc = grow_in_b(ctx, (msg_len ? msg_len : 1) * C)) return grc;
     cudaStream_t s = ctx->stream;
-    const bool resident = n <= C;  // one chunk: copied once, read by both passes
-    int rc = batch_verify_run(ctx, n, msg_len, [&](size_t off, size_t c, int pass, batch_rows &r) {
-        if (pass == 0 || !resident) {
-            CK(cudaMemcpyAsync(ctx->in_a, pkx + 32 * off, 32 * c, cudaMemcpyHostToDevice, s));
-            if (msg_len) CK(cudaMemcpyAsync(ctx->in_b, msg + msg_len * off, msg_len * c, cudaMemcpyHostToDevice, s));
-            CK(cudaMemcpyAsync(ctx->in_c, sig + 64 * off, 64 * c, cudaMemcpyHostToDevice, s));
-        }
-        r = batch_rows{ctx->in_a, ctx->in_b, ctx->in_c};
-        return S256_SUCCESS;
-    }, ctx->st, s);
+    int rc = batch_verify_host(ctx, pkx, msg, msg_len, sig, n);
     if (rc != S256_SUCCESS) return rc;
     CK(cudaMemcpyAsync(ok, ctx->st, 1, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));  // the one host synchronisation of the call
+    return check_launch(ctx);
+}
+// The batch equation of s256_schnorr_batch_verify as its kernels build it, copied back chunk by chunk.
+extern "C" int s256_debug_schnorr_batch_rows(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
+                                             const uint8_t *sig, size_t n, uint8_t *seed32, uint8_t *k64, uint8_t *pts128,
+                                             uint8_t *sum32, uint8_t *rejected) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    if (n == 0 || !pkx || (!msg && msg_len) || !sig || !seed32 || !k64 || !pts128 || !sum32 || !rejected)
+        return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    cudaStream_t s = ctx->stream;
+    std::vector<apt> aff;
+    int rc = batch_verify_host(ctx, pkx, msg, msg_len, sig, n, [&](size_t off, size_t c) {
+        aff.resize(2 * c);
+        CK(cudaMemcpyAsync(k64 + 64 * off, ctx->out, 64 * c, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(aff.data(), ctx->aff, 2 * c * sizeof(apt), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        for (size_t v = 0; v < 2 * c; v++) {
+            fe_to_be32(pts128 + 64 * (2 * off + v), aff[v].x);
+            fe_to_be32(pts128 + 64 * (2 * off + v) + 32, aff[v].y);
+        }
+        return S256_SUCCESS;
+    });
+    if (rc != S256_SUCCESS) return rc;
+    uint32_t seed[8], flag = 0;
+    CK(cudaMemcpyAsync(seed, ctx->bat + BAT_SEED, 32, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(sum32, ctx->bat + BAT_SUM_BE, 32, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(&flag, ctx->msm_flag, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    words_be32(seed32, seed);
+    *rejected = (uint8_t)(flag != 0);
     return check_launch(ctx);
 }
 
