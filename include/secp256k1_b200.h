@@ -202,6 +202,25 @@ int s256_schnorr_batch_verify(s256_ctx *ctx, const uint8_t *pkx32, const uint8_t
 int s256_schnorr_batch_verify_dev(s256_ctx *ctx, const uint8_t *d_pkx32, const uint8_t *d_msg, size_t msg_len,
                                   const uint8_t *d_sig64, size_t n, uint8_t *d_ok, void *stream);
 
+/* Recoverable ECDSA batch verification (per item: secec.PublicKey.Verify with EncodingCompactRecoverable,
+ * secec/ecdsa.go:221-227 -- RecoverPublicKey :244 on r||s||v, then a comparison with the key).  Rows: pk65
+ * (uncompressed keys), digest32 (leftmost 32 bytes of the digest, reduced mod n as in s256_ecdsa_verify) and sig65
+ * (r||s||v).  flags as for s256_ecdsa_verify (S256_FLAG_REJECT_MALLEABLE: s > n/2 fails).  *ok = 1 iff every row
+ * would verify; 0 otherwise (except with probability <= 2^-127 per call when some row is invalid).  n == 0 gives 1.
+ * Variable time (public data).
+ * One equation, (sum a_i u1_i) G + sum (a_i u2_i) Q_i - sum a_i R_i = O with R_i = RecoverPoint(r_i, v_i),
+ * u1_i = e_i / s_i, u2_i = r_i / s_i, a_0 = 1 and 128-bit a_i derived from a hash tree over all the rows (DESIGN.md),
+ * checked by one multi-scalar multiplication.  A row is rejected, and with it the batch, when r or s is not in [1, n),
+ * v >= 4, r + n >= p with v & 2, r (+ n) is not the x-coordinate of a curve point, the key does not decode as
+ * secec.NewPublicKey decodes it (04 || X || Y, canonical, on the curve), or, with S256_FLAG_REJECT_MALLEABLE, s > n/2.
+ * To find the invalid rows of a rejected batch, run s256_ecdsa_recover on it and compare each recovered key (status
+ * S256_ST_OK) with the row's key.  The _dev form writes the verdict byte to device memory and does not synchronise.
+ * S256_ERR_ARG for NULL arguments and for a context with max_batch < 2. */
+int s256_ecdsa_recoverable_batch_verify(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32, const uint8_t *sig65,
+                                        uint32_t flags, size_t n, uint8_t *ok);
+int s256_ecdsa_recoverable_batch_verify_dev(s256_ctx *ctx, const uint8_t *d_pk65, const uint8_t *d_digest32,
+                                            const uint8_t *d_sig65, uint32_t flags, size_t n, uint8_t *d_ok, void *stream);
+
 /* --- bitcoin.SchnorrPrivateKey.Sign (secec/bitcoin/schnorr.go:111-147 -> signSchnorr :322): BIP-340
  *     signing with caller-supplied auxiliary randomness (32 B per row; the reference draws it from
  *     its entropy source, :130-141).  priv32 as for NewPrivateKey; constant time. */
@@ -303,6 +322,11 @@ double s256_mac32_k_dsm(double adds_per_item, double beta_muls_per_item);
 int s256_debug_schnorr_batch_rows(s256_ctx *ctx, const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
                                   const uint8_t *sig64, size_t n, uint8_t *seed32, uint8_t *k64, uint8_t *pts128,
                                   uint8_t *sum32, uint8_t *rejected);
+/* The same for s256_ecdsa_recoverable_batch_verify: the seed; per row a_i and a_i u2_i mod n (k64) and the points
+ * -R_i and Q_i (pts128; G with scalar 0 for a rejected row); sum32 = sum a_i u1_i mod n; *rejected.  n >= 1. */
+int s256_debug_ecdsa_batch_rows(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32, const uint8_t *sig65,
+                                uint32_t flags, size_t n, uint8_t *seed32, uint8_t *k64, uint8_t *pts128, uint8_t *sum32,
+                                uint8_t *rejected);
 
 #if defined(__GNUC__)
 #pragma GCC visibility pop

@@ -37,13 +37,15 @@ EXPORTED_SYMBOLS = [
     "s256_new_public_keys", "s256_parse_asn1_public_keys_checked",
     "s256_ecdsa_verify_asn1", "s256_bitcoin_verify_asn1",
     "s256_ecdsa_recover", "s256_ecdsa_recover_dev",
+    "s256_ecdsa_recoverable_batch_verify", "s256_ecdsa_recoverable_batch_verify_dev",
     "s256_ecdsa_sign_rfc6979", "s256_ecdsa_sign_rfc6979_dev",
     "s256_schnorr_verify", "s256_schnorr_verify_dev", "s256_schnorr_sign", "s256_schnorr_sign_dev",
     "s256_schnorr_batch_verify", "s256_schnorr_batch_verify_dev",
     "s256_msm", "s256_msm_partial", "s256_msm_combine", "s256_msm_dev", "s256_msm_sharded", "s256_msm_sharded_dev",
     "s256_comm_unique_id", "s256_comm_init", "s256_comm_free", "s256_msm_plan", "s256_hash_to_curve", "s256_expand_message_xmd",
     "s256_debug_ladder_add_count", "s256_mac32_k_dsm",
-    "s256_debug_gen_table", "s256_debug_field_op", "s256_debug_schnorr_batch_rows", "s256_microbench_imad",
+    "s256_debug_gen_table", "s256_debug_field_op", "s256_debug_schnorr_batch_rows", "s256_debug_ecdsa_batch_rows",
+    "s256_microbench_imad",
     "s256_microbench_variant", "s256_microbench_fe_mul", "s256_profile_enable", "s256_profile_read",
     "s256_launch_count", "s256_mac32_per_item", "s256_host_alloc", "s256_host_free",
 ]
@@ -497,6 +499,32 @@ class Engine:
                     "ecdsa_recover")
         return out, st
 
+    # -- recoverable ECDSA batch verification: one verdict for the whole batch -----------------------
+    def ecdsa_recoverable_batch_verify(self, pk65, digest32, sig65, flags=0):
+        """True iff every r||s||v row recovers its key (PublicKey.Verify with EncodingCompactRecoverable,
+        secec/ecdsa.go:221-227), from one randomized multi-scalar multiplication; a batch with an invalid row is accepted
+        with probability <= 2^-127.  With CUDA tensors: a (1,) uint8 tensor, not synchronised."""
+        if _is_torch_cuda(pk65):
+            import torch
+            n = pk65.numel() // 65
+            if pk65.numel() != 65 * n or digest32.numel() != 32 * n or sig65.numel() != 65 * n:
+                raise ValueError("length mismatch")
+            ok = torch.empty(1, dtype=torch.uint8, device=pk65.device)
+            a = self._dev_args(pk65, digest32, sig65, ok)
+            self._check(self._lib.s256_ecdsa_recoverable_batch_verify_dev(self._ctx, a[0], a[1], a[2], C.c_uint32(flags),
+                                                                          C.c_size_t(n), a[3], self._stream()),
+                        "ecdsa_recoverable_batch_verify_dev")
+            return ok
+        pk, dg, sg = _host(pk65, 65), _host(digest32, 32), _host(sig65, 65)
+        n = len(pk)
+        if len(dg) != n or len(sg) != n:
+            raise ValueError("length mismatch")
+        ok = C.c_uint8(0)
+        self._check(self._lib.s256_ecdsa_recoverable_batch_verify(self._ctx, self._hp(pk), self._hp(dg), self._hp(sg),
+                                                                  C.c_uint32(flags), C.c_size_t(n), C.byref(ok)),
+                    "ecdsa_recoverable_batch_verify")
+        return bool(ok.value)
+
     # -- bitcoin.SchnorrPublicKey.Verify (secec/bitcoin/schnorr.go:221) --------
     def schnorr_verify(self, pkx32, msg, sig64):
         if _is_torch_cuda(pkx32):
@@ -716,6 +744,22 @@ class Engine:
                                                             self._hp(sg), C.c_size_t(n), self._hp(seed), self._hp(k),
                                                             self._hp(pts), self._hp(ssum), C.byref(rej)),
                     "debug_schnorr_batch_rows")
+        return seed.tobytes(), k, pts, ssum.tobytes(), bool(rej.value)
+
+    def debug_ecdsa_batch_rows(self, pk65, digest32, sig65, flags=0):
+        """What ecdsa_recoverable_batch_verify checks for these host rows: (seed (32,), k (n, 2, 32) = a_i and a_i u2_i
+        mod n, pts (n, 2, 64) = -R_i and Q_i as X||Y (G for a rejected row), sum (32,) = sum a_i u1_i mod n, rejected),
+        all big-endian bytes."""
+        pk, dg, sg = _host(pk65, 65), _host(digest32, 32), _host(sig65, 65)
+        n = len(pk)
+        if n == 0 or len(dg) != n or len(sg) != n:
+            raise ValueError("length mismatch or empty batch")
+        seed, k, pts, ssum, rej = (np.zeros(32, np.uint8), np.zeros((n, 2, 32), np.uint8), np.zeros((n, 2, 64), np.uint8),
+                                   np.zeros(32, np.uint8), C.c_uint8(0))
+        self._check(self._lib.s256_debug_ecdsa_batch_rows(self._ctx, self._hp(pk), self._hp(dg), self._hp(sg),
+                                                          C.c_uint32(flags), C.c_size_t(n), self._hp(seed), self._hp(k),
+                                                          self._hp(pts), self._hp(ssum), C.byref(rej)),
+                    "debug_ecdsa_batch_rows")
         return seed.tobytes(), k, pts, ssum.tobytes(), bool(rej.value)
 
     def profile_enable(self, on=True):

@@ -503,19 +503,37 @@ extern "C" int s256_msm_combine(s256_ctx *ctx, const uint8_t *partials96, size_t
 
 
 // ---------------------------------------------------------------------------
-// BIP-340 batch verification (batch.cuh): one verdict for a whole batch of Schnorr signatures, from one randomized
-// multi-scalar multiplication.
+// Batch verification (batch.cuh): one verdict for a whole batch of BIP-340 signatures or of recoverable ECDSA
+// signatures, from one randomized multi-scalar multiplication.
 //
 // Rows go in chunks of C = the largest power of two <= cap / 2, so that a chunk's 2C MSM points fit the per-chunk
 // scratch and the chunk roots are nodes of the batch's hash tree.  Pass 1 hashes the rows into leaves (ctx->u1) and
 // folds each chunk to its root (k_batch_tree); k_batch_seed folds the roots into the seed.  Pass 2 turns each chunk into
-// the 2c MSM rows (-R_i, a_i), (-P_i, a_i e_i) in ctx->aff / ctx->out plus per-CTA sums of a_i s_i (ctx->u1, folded into
-// one scalar by k_batch_fold) and runs them through the Pippenger body.  The finish adds (sum a_i s_i) G and tests the
-// sum for the identity.
+// its 2c MSM rows in ctx->aff / ctx->out plus per-CTA sums of the G-side scalars (ctx->u1, folded into one scalar by
+// k_batch_fold) and runs them through the Pippenger body.  The finish adds (the scalar sum) G and tests the sum for the
+// identity.  What differs between the two row kinds -- the leaf kernel, the prepare kernels and the seed's tag -- is a
+// kind struct (batch_schnorr, batch_ecdsa) the shared driver batch_verify_run is instantiated with.
 // ---------------------------------------------------------------------------
 constexpr int BATCH_SEG = 2 * S256_TPB;  // nodes one CTA of k_batch_tree folds into one
 // ctx->bat, in 32-bit words: the seed, the scalar sum (limbs), the scalar sum (big-endian bytes), one root per chunk
 constexpr size_t BAT_SEED = 0, BAT_SUM = 8, BAT_SUM_BE = 16, BAT_ROOTS = 24;
+
+// the sum of v over the CTA, valid in thread 0
+__device__ sc cta_sc_sum(sc v) {
+    __shared__ sc sh[S256_TPB];
+    const int t = threadIdx.x;
+    sh[t] = v;
+    __syncthreads();
+    for (int stride = S256_TPB / 2; stride >= 1; stride >>= 1) {
+        if (t < stride) {
+            sc a = sh[t], b = sh[t + stride];
+            sc_add(a, a, b);
+            sh[t] = a;
+        }
+        __syncthreads();
+    }
+    return sh[0];
+}
 
 __global__ void __launch_bounds__(S256_TPB) k_batch_leaves(const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
                                                            const uint8_t *sig64, size_t n, uint32_t *leaves) {
@@ -523,6 +541,16 @@ __global__ void __launch_bounds__(S256_TPB) k_batch_leaves(const uint8_t *pkx32,
     if (i >= n) return;
     uint32_t h[8];
     batch_leaf(h, pkx32 + 32 * i, sig64 + 64 * i, msg + msg_len * i, msg_len);
+    uint4 *o = reinterpret_cast<uint4 *>(leaves + 8 * i);
+    o[0] = make_uint4(h[0], h[1], h[2], h[3]);
+    o[1] = make_uint4(h[4], h[5], h[6], h[7]);
+}
+__global__ void __launch_bounds__(S256_TPB) k_ecdsa_batch_leaves(const uint8_t *pk65, const uint8_t *digest32,
+                                                                 const uint8_t *sig65, size_t n, uint32_t *leaves) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint32_t h[8];
+    batch_leaf_ecdsa(h, pk65 + 65 * i, digest32 + 32 * i, sig65 + 65 * i);
     uint4 *o = reinterpret_cast<uint4 *>(leaves + 8 * i);
     o[0] = make_uint4(h[0], h[1], h[2], h[3]);
     o[1] = make_uint4(h[4], h[5], h[6], h[7]);
@@ -561,19 +589,18 @@ __global__ void __launch_bounds__(S256_TPB) k_batch_tree(const uint32_t *in, siz
     if (t < 8) out[8 * (size_t)blockIdx.x + t] = sh[0][t];
 }
 // chunk roots -> seed (one thread; a batch has few chunks)
+template <class Kind>
 __global__ void k_batch_seed(uint32_t *bat, size_t chunks, uint64_t n) {
     if (blockIdx.x != 0 || threadIdx.x != 0) return;
     batch_tree_fold(bat + BAT_ROOTS, chunks);
-    batch_seed(bat + BAT_SEED, bat + BAT_ROOTS, n);
+    batch_seed(bat + BAT_SEED, bat + BAT_ROOTS, n, Kind::tag());
 }
 // rows [off, off + n) of the batch -> MSM rows 2i, 2i + 1 of the chunk, part[CTA] = the CTA's sum of a_i s_i,
 // flag |= a rejected row
 __global__ void __launch_bounds__(S256_TPB) k_batch_prepare(const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
                                                             const uint8_t *sig64, size_t n, size_t off, const uint32_t *seed_in,
                                                             apt *aff2, uint8_t *k2, sc *part, uint32_t *flag) {
-    __shared__ sc sh[S256_TPB];
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int t = threadIdx.x;
     sc as = sc_zero();
     if (i < n) {
         uint32_t seed[8];
@@ -582,39 +609,44 @@ __global__ void __launch_bounds__(S256_TPB) k_batch_prepare(const uint8_t *pkx32
                                          sig64 + 64 * i, seed, (uint64_t)(off + i));
         if (!ok) atomicOr(flag, 1u);
     }
-    sh[t] = as;
-    __syncthreads();
-    for (int stride = S256_TPB / 2; stride >= 1; stride >>= 1) {
-        if (t < stride) {
-            sc a = sh[t], b = sh[t + stride];
-            sc_add(a, a, b);
-            sh[t] = a;
-        }
-        __syncthreads();
+    sc sum = cta_sc_sum(as);
+    if (threadIdx.x == 0) part[blockIdx.x] = sum;
+}
+// ECDSA rows [0, n) of the chunk -> the points -R_i, Q_i of MSM rows 2i, 2i + 1 and pvalid[i], one row per thread
+__global__ void __launch_bounds__(S256_TPB) k_ecdsa_batch_points(const uint8_t *pk65, const uint8_t *sig65, size_t n,
+                                                                 apt *aff2, uint8_t *pvalid) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    pvalid[i] = (uint8_t)item_ecdsa_batch_points(aff2 + 2 * i, pk65 + 65 * i, sig65 + 65 * i);
+}
+// ECDSA rows [off, off + n) of the batch, K per thread sharing one inversion -> the scalars of MSM rows 2i, 2i + 1
+// (G with scalar 0 for a rejected row), part[CTA] = the CTA's sum of a_i u1_i, flag |= a rejected row
+template <int K>
+__global__ void __launch_bounds__(S256_TPB) k_ecdsa_batch_prepare(const uint8_t *digest32, const uint8_t *sig65,
+                                                                  uint32_t flags, const uint8_t *pvalid, size_t n, size_t off,
+                                                                  const uint32_t *seed_in, apt *aff2, uint8_t *k2, sc *part,
+                                                                  uint32_t *flag) {
+    const size_t stride = (n + K - 1) / K;
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    sc au1 = sc_zero();
+    if (t < stride) {
+        uint32_t seed[8];
+        for (int k = 0; k < 8; k++) seed[k] = seed_in[k];
+        uint32_t ok = group_ecdsa_batch_prepare<K>(t, stride, n, off, digest32, sig65, flags, pvalid, seed, aff2, k2, au1);
+        if (!ok) atomicOr(flag, 1u);
     }
-    if (t == 0) part[blockIdx.x] = sh[0];
+    sc sum = cta_sc_sum(au1);
+    if (threadIdx.x == 0) part[blockIdx.x] = sum;
 }
 // the scalar sum (+)= the m CTA sums (first = overwrite), kept as limbs and as big-endian bytes.  One CTA.
 __global__ void __launch_bounds__(S256_TPB) k_batch_fold(const sc *part, size_t m, uint32_t *bat, int first) {
-    __shared__ sc sh[S256_TPB];
-    const int t = threadIdx.x;
     sc acc = sc_zero();
-    for (size_t j = t; j < m; j += S256_TPB) {
+    for (size_t j = threadIdx.x; j < m; j += S256_TPB) {
         sc q = part[j];
         sc_add(acc, acc, q);
     }
-    sh[t] = acc;
-    __syncthreads();
-    for (int stride = S256_TPB / 2; stride >= 1; stride >>= 1) {
-        if (t < stride) {
-            sc a = sh[t], b = sh[t + stride];
-            sc_add(a, a, b);
-            sh[t] = a;
-        }
-        __syncthreads();
-    }
-    if (t == 0) {
-        sc r = sh[0];
+    sc r = cta_sc_sum(acc);
+    if (threadIdx.x == 0) {
         sc *sum = reinterpret_cast<sc *>(bat + BAT_SUM);
         if (!first) {
             sc a = *sum;
@@ -646,15 +678,52 @@ static int batch_ensure(s256_ctx *ctx, size_t chunks) {
     ctx->bat_chunks = chunks;
     return S256_SUCCESS;
 }
+// A batch's rows: three arrays of fixed-width rows (width 0: no bytes) and the flags of the call.
+//   BIP-340: a = x-only keys (32), b = messages (msg_len), c = r||s (64)
+//   ECDSA:   a = keys (65),        b = digests (32),       c = r||s||v (65)
 struct batch_rows {
-    const uint8_t *pkx, *msg, *sig;
+    const uint8_t *a, *b, *c;
+    size_t wa, wb, wc;
+    uint32_t flags;
+    batch_rows at(size_t off) const { return {a + wa * off, wb ? b + wb * off : b, c + wc * off, wa, wb, wc, flags}; }
 };
-// chunk_done(off, c): called once per chunk while its MSM rows are in ctx->out / ctx->aff (s256_debug_schnorr_batch_rows)
+// The row kinds: the seed's tag, pass 1 (leaves of c rows into `leaves`) and pass 2 (the chunk's MSM rows and per-CTA
+// G-side sums in ctx->u1; returns the number of CTA sums).
+struct batch_schnorr {
+    static __host__ __device__ const char *tag() { return S256_BATCH_TAG_BIP340; }
+    static void leaves(s256_ctx *ctx, const batch_rows &r, size_t c, uint32_t *leaves, cudaStream_t s) {
+        LAUNCH(ctx, k_batch_leaves, grid_for(c), 0, s, r.a, r.b, r.wb, r.c, c, leaves);
+    }
+    static size_t prepare(s256_ctx *ctx, const batch_rows &r, size_t c, size_t off, cudaStream_t s) {
+        LAUNCH(ctx, k_batch_prepare, grid_for(c), 0, s, r.a, r.b, r.wb, r.c, c, off, ctx->bat + BAT_SEED, ctx->aff, ctx->out,
+               ctx->u1, ctx->msm_flag);
+        return grid_for(c);
+    }
+};
+struct batch_ecdsa {
+    static __host__ __device__ const char *tag() { return S256_BATCH_TAG_ECDSA; }
+    static void leaves(s256_ctx *ctx, const batch_rows &r, size_t c, uint32_t *leaves, cudaStream_t s) {
+        LAUNCH(ctx, k_ecdsa_batch_leaves, grid_for(c), 0, s, r.a, r.b, r.c, c, leaves);
+    }
+    // The points go one row per thread; the scalars K rows per thread (inv_k_for), so that K rows share the inversion
+    // of s without running the square root of RecoverPoint on c / K threads.
+    static size_t prepare(s256_ctx *ctx, const batch_rows &r, size_t c, size_t off, cudaStream_t s) {
+        LAUNCH(ctx, k_ecdsa_batch_points, grid_for(c), 0, s, r.a, r.c, c, ctx->aff, ctx->pvalid);
+        size_t parts = 0;
+        DISPATCH_K(c, {
+            LAUNCH(ctx, k_ecdsa_batch_prepare<KK>, grid_for_groups(c, KK), 0, s, r.b, r.c, r.flags, ctx->pvalid, c, off,
+                   ctx->bat + BAT_SEED, ctx->aff, ctx->out, ctx->u1, ctx->msm_flag);
+            parts = grid_for_groups(c, KK);
+        });
+        return parts;
+    }
+};
+// chunk_done(off, c): called once per chunk while its MSM rows are in ctx->out / ctx->aff (the debug hooks)
 using batch_chunk_fn = std::function<int(size_t, size_t)>;
 // n >= 1 rows; rows(off, c, pass, r) gives the device rows of a chunk (the host form copies them in first).
 // The verdict byte goes to d_ok; nothing is synchronised unless chunk_done does.
-template <typename F>
-static int batch_verify_run(s256_ctx *ctx, size_t n, size_t msg_len, F rows, uint8_t *d_ok, cudaStream_t s,
+template <class Kind, typename F>
+static int batch_verify_run(s256_ctx *ctx, size_t n, F rows, uint8_t *d_ok, cudaStream_t s,
                             const batch_chunk_fn &chunk_done = nullptr) {
     int rc = msm_ensure(ctx);
     if (rc != S256_SUCCESS) return rc;
@@ -670,7 +739,7 @@ static int batch_verify_run(s256_ctx *ctx, size_t n, size_t msg_len, F rows, uin
         const size_t off = k * C, c = n - off < C ? n - off : C;
         rc = rows(off, c, 0, r);
         if (rc != S256_SUCCESS) return rc;
-        LAUNCH(ctx, k_batch_leaves, grid_for(c), 0, s, r.pkx, r.msg, msg_len, r.sig, c, leaves);
+        Kind::leaves(ctx, r, c, leaves, s);
         const uint32_t *src = leaves;
         size_t m = c;
         int side = 0;
@@ -683,7 +752,7 @@ static int batch_verify_run(s256_ctx *ctx, size_t n, size_t msg_len, F rows, uin
             m = g;
         } while (m > 1);
     }
-    k_batch_seed<<<1, 1, 0, s>>>(ctx->bat, chunks, (uint64_t)n);
+    k_batch_seed<Kind><<<1, 1, 0, s>>>(ctx->bat, chunks, (uint64_t)n);
     ctx->launches.fetch_add(1, std::memory_order_relaxed);
     // pass 2: per chunk, the MSM rows and the scalar sum, then the Pippenger body
     CK(cudaMemsetAsync(ctx->msm_flag, 0, 4, s));
@@ -691,15 +760,14 @@ static int batch_verify_run(s256_ctx *ctx, size_t n, size_t msg_len, F rows, uin
         const size_t off = k * C, c = n - off < C ? n - off : C;
         rc = rows(off, c, 1, r);
         if (rc != S256_SUCCESS) return rc;
-        LAUNCH(ctx, k_batch_prepare, grid_for(c), 0, s, r.pkx, r.msg, msg_len, r.sig, c, off, ctx->bat + BAT_SEED, ctx->aff,
-               ctx->out, ctx->u1, ctx->msm_flag);
-        k_batch_fold<<<1, S256_TPB, 0, s>>>(ctx->u1, (size_t)grid_for(c), ctx->bat, k == 0);
+        const size_t parts = Kind::prepare(ctx, r, c, off, s);
+        k_batch_fold<<<1, S256_TPB, 0, s>>>(ctx->u1, parts, ctx->bat, k == 0);
         ctx->launches.fetch_add(1, std::memory_order_relaxed);
         if (chunk_done && (rc = chunk_done(off, c)) != S256_SUCCESS) return rc;
         rc = chunk_msm_body(ctx, ctx->out, 2 * c, 1, k == 0, s);
         if (rc != S256_SUCCESS) return rc;
     }
-    // finish: + (sum a_i s_i) G, then the verdict
+    // finish: + (the scalar sum) G, then the verdict
     s256_launch_base_mult_ct(reinterpret_cast<const uint8_t *>(ctx->bat + BAT_SUM_BE), 1, ctx->ct_tab, ctx->ct_tab_small,
                              ctx->ct_tab_huge, ctx->res, s);
     k_acc_point<<<1, 1, 0, s>>>(ctx->res, ctx->msm_acc, 0);
@@ -707,69 +775,59 @@ static int batch_verify_run(s256_ctx *ctx, size_t n, size_t msg_len, F rows, uin
     ctx->launches.fetch_add(3, std::memory_order_relaxed);
     return check_launch(ctx);
 }
-extern "C" int s256_schnorr_batch_verify_dev(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
-                                             const uint8_t *sig, size_t n, uint8_t *ok, void *stream) {
-    ENTER(ctx);
-    if (!ok || (n && (!pkx || (!msg && msg_len) || !sig))) return S256_ERR_ARG;
-    if (ctx->cap < 2) return S256_ERR_ARG;  // a chunk needs two MSM rows per signature
-    cudaStream_t s = (cudaStream_t)stream;
-    scratch_guard sg_(ctx, s, false);
+// The device form: rows in device memory, the verdict byte to d_ok, nothing synchronised.
+template <class Kind>
+static int batch_verify_dev(s256_ctx *ctx, const batch_rows &dev, size_t n, uint8_t *d_ok, cudaStream_t s) {
     if (n == 0) {
-        CK(cudaMemsetAsync(ok, 1, 1, s));
+        CK(cudaMemsetAsync(d_ok, 1, 1, s));
         return S256_SUCCESS;
     }
-    return batch_verify_run(ctx, n, msg_len, [&](size_t off, size_t, int, batch_rows &r) {
-        r = batch_rows{pkx + 32 * off, msg_len ? msg + msg_len * off : msg, sig + 64 * off};
+    return batch_verify_run<Kind>(ctx, n, [&](size_t off, size_t, int, batch_rows &r) {
+        r = dev.at(off);
         return S256_SUCCESS;
-    }, ok, s);
+    }, d_ok, s);
 }
 // The host form's rows: a batch of one chunk is copied in once and read by both passes, a longer one chunk by chunk in
 // each pass.  The verdict byte goes to ctx->st.
-static int batch_verify_host(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len, const uint8_t *sig,
-                             size_t n, const batch_chunk_fn &chunk_done = nullptr) {
+template <class Kind>
+static int batch_verify_host(s256_ctx *ctx, const batch_rows &host, size_t n, const batch_chunk_fn &chunk_done = nullptr) {
     const size_t C = batch_chunk(ctx);
-    if (int grc = grow_in_b(ctx, (msg_len ? msg_len : 1) * C)) return grc;
+    if (int grc = grow_in_b(ctx, (host.wb ? host.wb : 1) * C)) return grc;
     cudaStream_t s = ctx->stream;
     const bool resident = n <= C;
-    return batch_verify_run(ctx, n, msg_len, [&](size_t off, size_t c, int pass, batch_rows &r) {
+    const batch_rows staged{ctx->in_a, ctx->in_b, ctx->in_c, host.wa, host.wb, host.wc, host.flags};
+    return batch_verify_run<Kind>(ctx, n, [&](size_t off, size_t c, int pass, batch_rows &r) {
         if (pass == 0 || !resident) {
-            CK(cudaMemcpyAsync(ctx->in_a, pkx + 32 * off, 32 * c, cudaMemcpyHostToDevice, s));
-            if (msg_len) CK(cudaMemcpyAsync(ctx->in_b, msg + msg_len * off, msg_len * c, cudaMemcpyHostToDevice, s));
-            CK(cudaMemcpyAsync(ctx->in_c, sig + 64 * off, 64 * c, cudaMemcpyHostToDevice, s));
+            const batch_rows h = host.at(off);
+            CK(cudaMemcpyAsync(ctx->in_a, h.a, h.wa * c, cudaMemcpyHostToDevice, s));
+            if (h.wb) CK(cudaMemcpyAsync(ctx->in_b, h.b, h.wb * c, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(ctx->in_c, h.c, h.wc * c, cudaMemcpyHostToDevice, s));
         }
-        r = batch_rows{ctx->in_a, ctx->in_b, ctx->in_c};
+        r = staged;
         return S256_SUCCESS;
     }, ctx->st, s, chunk_done);
 }
-extern "C" int s256_schnorr_batch_verify(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
-                                         const uint8_t *sig, size_t n, uint8_t *ok) {
-    ENTER(ctx);
-    scratch_guard sg_(ctx, ctx->stream, true);
-    if (!ok || (n && (!pkx || (!msg && msg_len) || !sig))) return S256_ERR_ARG;
-    if (ctx->cap < 2) return S256_ERR_ARG;
+// host rows -> *ok, the one host synchronisation of the call
+template <class Kind>
+static int batch_verify_host_sync(s256_ctx *ctx, const batch_rows &host, size_t n, uint8_t *ok) {
     if (n == 0) {
         *ok = 1;
         return S256_SUCCESS;
     }
     cudaStream_t s = ctx->stream;
-    int rc = batch_verify_host(ctx, pkx, msg, msg_len, sig, n);
+    int rc = batch_verify_host<Kind>(ctx, host, n);
     if (rc != S256_SUCCESS) return rc;
     CK(cudaMemcpyAsync(ok, ctx->st, 1, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));  // the one host synchronisation of the call
+    CK(cudaStreamSynchronize(s));
     return check_launch(ctx);
 }
-// The batch equation of s256_schnorr_batch_verify as its kernels build it, copied back chunk by chunk.
-extern "C" int s256_debug_schnorr_batch_rows(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
-                                             const uint8_t *sig, size_t n, uint8_t *seed32, uint8_t *k64, uint8_t *pts128,
-                                             uint8_t *sum32, uint8_t *rejected) {
-    ENTER(ctx);
-    scratch_guard sg_(ctx, ctx->stream, true);
-    if (n == 0 || !pkx || (!msg && msg_len) || !sig || !seed32 || !k64 || !pts128 || !sum32 || !rejected)
-        return S256_ERR_ARG;
-    if (ctx->cap < 2) return S256_ERR_ARG;
+// The batch equation as the kernels build it, copied back chunk by chunk (the s256_debug_*_batch_rows hooks).
+template <class Kind>
+static int batch_debug_rows(s256_ctx *ctx, const batch_rows &host, size_t n, uint8_t *seed32, uint8_t *k64,
+                            uint8_t *pts128, uint8_t *sum32, uint8_t *rejected) {
     cudaStream_t s = ctx->stream;
     std::vector<apt> aff;
-    int rc = batch_verify_host(ctx, pkx, msg, msg_len, sig, n, [&](size_t off, size_t c) {
+    int rc = batch_verify_host<Kind>(ctx, host, n, [&](size_t off, size_t c) {
         aff.resize(2 * c);
         CK(cudaMemcpyAsync(k64 + 64 * off, ctx->out, 64 * c, cudaMemcpyDeviceToHost, s));
         CK(cudaMemcpyAsync(aff.data(), ctx->aff, 2 * c * sizeof(apt), cudaMemcpyDeviceToHost, s));
@@ -789,6 +847,69 @@ extern "C" int s256_debug_schnorr_batch_rows(s256_ctx *ctx, const uint8_t *pkx, 
     words_be32(seed32, seed);
     *rejected = (uint8_t)(flag != 0);
     return check_launch(ctx);
+}
+
+static batch_rows schnorr_rows(const uint8_t *pkx, const uint8_t *msg, size_t msg_len, const uint8_t *sig) {
+    return {pkx, msg, sig, 32, msg_len, 64, 0u};
+}
+extern "C" int s256_schnorr_batch_verify_dev(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
+                                             const uint8_t *sig, size_t n, uint8_t *ok, void *stream) {
+    ENTER(ctx);
+    if (!ok || (n && (!pkx || (!msg && msg_len) || !sig))) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;  // a chunk needs two MSM rows per signature
+    cudaStream_t s = (cudaStream_t)stream;
+    scratch_guard sg_(ctx, s, false);
+    return batch_verify_dev<batch_schnorr>(ctx, schnorr_rows(pkx, msg, msg_len, sig), n, ok, s);
+}
+extern "C" int s256_schnorr_batch_verify(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
+                                         const uint8_t *sig, size_t n, uint8_t *ok) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    if (!ok || (n && (!pkx || (!msg && msg_len) || !sig))) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    return batch_verify_host_sync<batch_schnorr>(ctx, schnorr_rows(pkx, msg, msg_len, sig), n, ok);
+}
+extern "C" int s256_debug_schnorr_batch_rows(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
+                                             const uint8_t *sig, size_t n, uint8_t *seed32, uint8_t *k64, uint8_t *pts128,
+                                             uint8_t *sum32, uint8_t *rejected) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    if (n == 0 || !pkx || (!msg && msg_len) || !sig || !seed32 || !k64 || !pts128 || !sum32 || !rejected)
+        return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    return batch_debug_rows<batch_schnorr>(ctx, schnorr_rows(pkx, msg, msg_len, sig), n, seed32, k64, pts128, sum32, rejected);
+}
+
+static batch_rows ecdsa_rows(const uint8_t *pk65, const uint8_t *digest32, const uint8_t *sig65, uint32_t flags) {
+    return {pk65, digest32, sig65, 65, 32, 65, flags};
+}
+extern "C" int s256_ecdsa_recoverable_batch_verify_dev(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32,
+                                                       const uint8_t *sig65, uint32_t flags, size_t n, uint8_t *ok,
+                                                       void *stream) {
+    ENTER(ctx);
+    if (!ok || (n && (!pk65 || !digest32 || !sig65))) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    scratch_guard sg_(ctx, s, false);
+    return batch_verify_dev<batch_ecdsa>(ctx, ecdsa_rows(pk65, digest32, sig65, flags), n, ok, s);
+}
+extern "C" int s256_ecdsa_recoverable_batch_verify(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32,
+                                                   const uint8_t *sig65, uint32_t flags, size_t n, uint8_t *ok) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    if (!ok || (n && (!pk65 || !digest32 || !sig65))) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    return batch_verify_host_sync<batch_ecdsa>(ctx, ecdsa_rows(pk65, digest32, sig65, flags), n, ok);
+}
+extern "C" int s256_debug_ecdsa_batch_rows(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32, const uint8_t *sig65,
+                                           uint32_t flags, size_t n, uint8_t *seed32, uint8_t *k64, uint8_t *pts128,
+                                           uint8_t *sum32, uint8_t *rejected) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    if (n == 0 || !pk65 || !digest32 || !sig65 || !seed32 || !k64 || !pts128 || !sum32 || !rejected) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    return batch_debug_rows<batch_ecdsa>(ctx, ecdsa_rows(pk65, digest32, sig65, flags), n, seed32, k64, pts128, sum32,
+                                         rejected);
 }
 
 

@@ -90,6 +90,27 @@ func (e *Engine) RecoverPublicKeyBatch(digest32, sig65 []byte) (pk65 []byte, sta
 	return
 }
 
+// ECDSARecoverableBatchVerify is recoverable ECDSA batch verification: true iff every row of uncompressed key (65 B),
+// digest (32 B) and r||s||v (65 B) would pass secec.PublicKey.Verify with EncodingCompactRecoverable
+// (secec/ecdsa.go:221-227), from one randomized multi-scalar multiplication; a batch with an invalid row passes with
+// probability <= 2^-127.  rejectMalleable is ECDSAOptions.RejectMalleable.  RecoverPublicKeyBatch and a comparison
+// with the keys find the bad rows of a rejected batch.
+func (e *Engine) ECDSARecoverableBatchVerify(pk65, digest32, sig65 []byte, rejectMalleable bool) (bool, error) {
+	n := len(pk65) / 65
+	if len(pk65) != 65*n || len(digest32) != 32*n || len(sig65) != 65*n {
+		panic("secp256k1b200: ECDSARecoverableBatchVerify: length mismatch")
+	}
+	var flags C.uint32_t
+	if rejectMalleable {
+		flags = C.S256_FLAG_REJECT_MALLEABLE
+	}
+	var ok C.uint8_t
+	if err := e.err(C.s256_ecdsa_recoverable_batch_verify(e.ctx, ptr(pk65), ptr(digest32), ptr(sig65), flags, C.size_t(n), &ok)); err != nil {
+		return false, err
+	}
+	return ok == 1, nil
+}
+
 // SignRFC6979Batch is PrivateKey.Sign(secec.RFC6979SHA256(), digest, EncodingCompactRecoverable) over rows of
 // private scalars (32 B) and digests (32 B): returns r||s rows (low-s), recovery ids and per-row status.
 func (e *Engine) SignRFC6979Batch(priv32, digest32 []byte) (sig64, recid, status []byte, err error) {

@@ -664,6 +664,18 @@ inline void RecoverPublicKeyBatch(const uint8_t *digest32, const uint8_t *sig65,
                                   Engine &e = Engine::Default()) {
     e.check(s256_ecdsa_recover(e.ctx(), digest32, sig65, n, pk65, status), "RecoverPublicKeyBatch");
 }
+// Recoverable ECDSA batch verification: true iff every row would pass PublicKey::Verify with
+// EncodingCompactRecoverable (ecdsa.go:221-227; reject_malleable as ECDSAOptions::RejectMalleable), from one randomized
+// multi-scalar multiplication; a batch with an invalid row passes with probability <= 2^-127.  RecoverPublicKeyBatch
+// and a comparison with the keys find the bad rows.
+inline bool RecoverableBatchVerify(const uint8_t *pk65, const uint8_t *digest32, const uint8_t *sig65, size_t n,
+                                   bool reject_malleable = false, Engine &e = Engine::Default()) {
+    uint8_t ok = 0;
+    e.check(s256_ecdsa_recoverable_batch_verify(e.ctx(), pk65, digest32, sig65,
+                                                reject_malleable ? S256_FLAG_REJECT_MALLEABLE : 0u, n, &ok),
+            "RecoverableBatchVerify");
+    return ok == 1;
+}
 inline void ECDHBatch(const uint8_t *k32, const uint8_t *pt65, size_t n, uint8_t *x32, uint8_t *status, Engine &e = Engine::Default()) {
     e.check(s256_ecdh(e.ctx(), k32, pt65, n, x32, status), "ECDHBatch");
 }

@@ -52,14 +52,10 @@ def tagged_hash(tag, data):
     return hashlib.sha256(t + t + data).digest()
 
 
-def ecdsa_batch(n, base_mult, start=0, seed=SEED, corrupt_every=16):
-    """Config 2: returns dict(pk65, digest32, sig64, expected) as uint8 arrays.
-
-    d_i = D("key", i) mod n != 0, Q_i = d_i*G, z_i = D("msg", i),
-    k_i = D("nonce", i) mod n != 0, r = x(k*G) mod n, s = (z + r*d)/k,
-    low-s normalised for even i only; every `corrupt_every`-th item corrupted,
-    cycling: one bit of r / of s / of z flipped, Q replaced by Q_{i-1}.
-    `expected` is by construction (valid unless corrupted)."""
+def _ecdsa_signatures(n, base_mult, start, seed):
+    """d_i = D("key", i) mod n != 0, Q_i = d_i*G, z_i = D("msg", i), k_i = D("nonce", i) mod n != 0, r = x(k*G) mod n,
+    s = (z + r*d)/k, low-s normalised for even i only -> (pk65, digest32, sig64, recovery ids) as uint8 arrays; the
+    recovery id is the parity of y(kG), + 2 when x(kG) >= n, and flips with the sign of s."""
     d = [_nonzero_mod_n(x) for x in _stream_ints(b"key", start, n, seed)]
     k = [_nonzero_mod_n(x) for x in _stream_ints(b"nonce", start, n, seed)]
     zb = [D(b"msg", start + i, seed) for i in range(n)]
@@ -71,18 +67,35 @@ def ecdsa_batch(n, base_mult, start=0, seed=SEED, corrupt_every=16):
     kg = np.asarray(kg, dtype=np.uint8).reshape(n, 65)
     kinv = batch_inverse_mod_n(k)
     sig = np.zeros((n, 64), np.uint8)
+    recid = np.zeros(n, np.uint8)
     digest = np.frombuffer(b"".join(zb), np.uint8).reshape(n, 32).copy()
-    expected = np.ones(n, np.uint8)
     for i in range(n):
         gi = start + i
-        r = int.from_bytes(kg[i, 1:33].tobytes(), "big") % N
+        x = int.from_bytes(kg[i, 1:33].tobytes(), "big")
+        r = x % N
         z = int.from_bytes(zb[i], "big") % N
         s = kinv[i] * (z + r * d[i]) % N
+        v = (kg[i, 64] & 1) | (2 if x >= N else 0)
         if gi % 2 == 0 and s > N // 2:
             s = N - s
+            v ^= 1
         assert r != 0 and s != 0
         sig[i, :32] = np.frombuffer(r.to_bytes(32, "big"), np.uint8)
         sig[i, 32:] = np.frombuffer(s.to_bytes(32, "big"), np.uint8)
+        recid[i] = v
+    return pk, digest, sig, recid
+
+
+def ecdsa_batch(n, base_mult, start=0, seed=SEED, corrupt_every=16):
+    """Config 2: returns dict(pk65, digest32, sig64, expected) as uint8 arrays.
+
+    d_i = D("key", i) mod n != 0, Q_i = d_i*G, z_i = D("msg", i),
+    k_i = D("nonce", i) mod n != 0, r = x(k*G) mod n, s = (z + r*d)/k,
+    low-s normalised for even i only; every `corrupt_every`-th item corrupted,
+    cycling: one bit of r / of s / of z flipped, Q replaced by Q_{i-1}.
+    `expected` is by construction (valid unless corrupted)."""
+    pk, digest, sig, _ = _ecdsa_signatures(n, base_mult, start, seed)
+    expected = np.ones(n, np.uint8)
     if corrupt_every:
         pk_orig = pk.copy()
         for i in range(n):
@@ -104,6 +117,37 @@ def ecdsa_batch(n, base_mult, start=0, seed=SEED, corrupt_every=16):
                     pk[i] = pk_orig[i - 1]
             expected[i] = 0
     return {"pk65": pk, "digest32": digest, "sig64": sig, "expected": expected}
+
+
+def ecdsa_recoverable_batch(n, base_mult, start=0, seed=SEED, corrupt_every=16):
+    """The signatures of ecdsa_batch as recoverable r||s||v rows (secec EncodingCompactRecoverable): returns
+    dict(pk65, digest32, sig65, expected).  v is the parity of y(kG) (+ 2 when x(kG) >= n), flipped where s was low-s
+    normalised (even i), so every uncorrupted row recovers its key; odd rows keep a high s about half the time and fail
+    under S256_FLAG_REJECT_MALLEABLE.  Every `corrupt_every`-th row is corrupted, cycling: one bit of r / of s / of z
+    flipped, Q replaced by Q_{i-1}, v ^= 1."""
+    pk, digest, sig, recid = _ecdsa_signatures(n, base_mult, start, seed)
+    sig65 = np.concatenate([sig, recid.reshape(n, 1)], axis=1)
+    expected = np.ones(n, np.uint8)
+    if corrupt_every:
+        pk_orig = pk.copy()
+        for i in range(n):
+            gi = start + i
+            if gi % corrupt_every != corrupt_every - 1:
+                continue
+            kind = (gi // corrupt_every) % 5
+            bit = gi % 250
+            if kind == 0:
+                sig65[i, 31 - bit // 8] ^= 1 << (bit % 8)
+            elif kind == 1:
+                sig65[i, 63 - bit // 8] ^= 1 << (bit % 8)
+            elif kind == 2:
+                digest[i, 31 - bit // 8] ^= 1 << (bit % 8)
+            elif kind == 3 and i > 0:
+                pk[i] = pk_orig[i - 1]
+            else:
+                sig65[i, 64] ^= 1
+            expected[i] = 0
+    return {"pk65": pk, "digest32": digest, "sig65": sig65, "expected": expected}
 
 
 def schnorr_batch(n, base_mult, start=0, seed=SEED, corrupt_every=16):
