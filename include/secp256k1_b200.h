@@ -229,6 +229,37 @@ int s256_schnorr_sign(s256_ctx *ctx, const uint8_t *priv32, const uint8_t *msg, 
 int s256_schnorr_sign_dev(s256_ctx *ctx, const uint8_t *d_priv32, const uint8_t *d_msg, size_t msg_len,
                           const uint8_t *d_aux32, size_t n, uint8_t *d_sig64, uint8_t *d_status, void *stream);
 
+/* --- BIP-340 over messages of different lengths (bitcoin.SchnorrPublicKey.Verify, schnorr.go:221, and
+ *     bitcoin.SchnorrPrivateKey.Sign, :111, take a message of any length; BIP-340 allows it since 2022).
+ *     Messages arrive concatenated in `msg` as for s256_parse_asn1_signatures: row i is
+ *     msg[offsets[i] .. offsets[i+1]), n + 1 offsets (offsets[0] need not be 0); msg may be NULL when every row is
+ *     empty (host forms only).  Every other buffer is laid out as for the uniform twin.
+ *   s256_schnorr_verify_varlen: ok[i] as s256_schnorr_verify gives it for row i alone.
+ *   s256_schnorr_batch_verify_varlen: the verdict of s256_schnorr_batch_verify (the same equation, soundness bound,
+ *     rejection rules and max_batch < 2 rule) over these rows.  The randomizers are defined as for the uniform call,
+ *     so rows that all have length L give the seed and rows of the uniform call with msg_len = L.
+ *   s256_schnorr_sign_varlen: sig64 and status as s256_schnorr_sign gives them for each row.
+ *   s256_debug_schnorr_batch_rows_varlen: the outputs of s256_debug_schnorr_batch_rows.
+ * The host forms return S256_ERR_ARG for decreasing offsets, checked before anything is enqueued, and S256_ERR_NOMEM
+ * when the message bytes of one chunk (max_batch rows) do not fit the device staging.  In the _dev forms offsets is a
+ * device array of n + 1 values relative to the device pointer msg; these forms cannot check it without synchronising,
+ * so a row with offsets[i+1] < offsets[i] is invalid and none of its message bytes are read: ok[i] = 0, the batch
+ * verdict 0, the sign status S256_ST_INVALID (zeroed signature).  One thread hashes one row: a warp waits for its
+ * longest message, so a very long message slows the 31 rows beside it. */
+int s256_schnorr_verify_varlen(s256_ctx *ctx, const uint8_t *pkx32, const uint8_t *msg, const size_t *offsets,
+                               const uint8_t *sig64, size_t n, uint8_t *ok);
+int s256_schnorr_verify_varlen_dev(s256_ctx *ctx, const uint8_t *d_pkx32, const uint8_t *d_msg, const size_t *d_offsets,
+                                   const uint8_t *d_sig64, size_t n, uint8_t *d_ok, void *stream);
+int s256_schnorr_batch_verify_varlen(s256_ctx *ctx, const uint8_t *pkx32, const uint8_t *msg, const size_t *offsets,
+                                     const uint8_t *sig64, size_t n, uint8_t *ok);
+int s256_schnorr_batch_verify_varlen_dev(s256_ctx *ctx, const uint8_t *d_pkx32, const uint8_t *d_msg,
+                                         const size_t *d_offsets, const uint8_t *d_sig64, size_t n, uint8_t *d_ok,
+                                         void *stream);
+int s256_schnorr_sign_varlen(s256_ctx *ctx, const uint8_t *priv32, const uint8_t *msg, const size_t *offsets,
+                             const uint8_t *aux32, size_t n, uint8_t *sig64, uint8_t *status);
+int s256_schnorr_sign_varlen_dev(s256_ctx *ctx, const uint8_t *d_priv32, const uint8_t *d_msg, const size_t *d_offsets,
+                                 const uint8_t *d_aux32, size_t n, uint8_t *d_sig64, uint8_t *d_status, void *stream);
+
 /* --- h2c.Secp256k1_XMD_SHA256_SSWU_RO / _NU (secec/h2c/h2c.go:25,49): RFC 9380 hash_to_curve
  *     (random_oracle != 0) or encode_to_curve over n messages of msg_len bytes sharing one domain
  *     separation tag.  dst_len == 0 is an error (errInvalidDomainSep); a DST longer than 255 bytes is
@@ -322,6 +353,10 @@ double s256_mac32_k_dsm(double adds_per_item, double beta_muls_per_item);
 int s256_debug_schnorr_batch_rows(s256_ctx *ctx, const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
                                   const uint8_t *sig64, size_t n, uint8_t *seed32, uint8_t *k64, uint8_t *pts128,
                                   uint8_t *sum32, uint8_t *rejected);
+/* The same over messages of different lengths, laid out as for s256_schnorr_batch_verify_varlen. */
+int s256_debug_schnorr_batch_rows_varlen(s256_ctx *ctx, const uint8_t *pkx32, const uint8_t *msg, const size_t *offsets,
+                                         const uint8_t *sig64, size_t n, uint8_t *seed32, uint8_t *k64, uint8_t *pts128,
+                                         uint8_t *sum32, uint8_t *rejected);
 /* The same for s256_ecdsa_recoverable_batch_verify: the seed; per row a_i and a_i u2_i mod n (k64) and the points
  * -R_i and Q_i (pts128; G with scalar 0 for a rejected row); sum32 = sum a_i u1_i mod n; *rejected.  n >= 1. */
 int s256_debug_ecdsa_batch_rows(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32, const uint8_t *sig65,

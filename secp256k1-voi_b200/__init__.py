@@ -41,6 +41,9 @@ EXPORTED_SYMBOLS = [
     "s256_ecdsa_sign_rfc6979", "s256_ecdsa_sign_rfc6979_dev",
     "s256_schnorr_verify", "s256_schnorr_verify_dev", "s256_schnorr_sign", "s256_schnorr_sign_dev",
     "s256_schnorr_batch_verify", "s256_schnorr_batch_verify_dev",
+    "s256_schnorr_verify_varlen", "s256_schnorr_verify_varlen_dev", "s256_schnorr_batch_verify_varlen",
+    "s256_schnorr_batch_verify_varlen_dev", "s256_schnorr_sign_varlen", "s256_schnorr_sign_varlen_dev",
+    "s256_debug_schnorr_batch_rows_varlen",
     "s256_msm", "s256_msm_partial", "s256_msm_combine", "s256_msm_dev", "s256_msm_sharded", "s256_msm_sharded_dev",
     "s256_comm_unique_id", "s256_comm_init", "s256_comm_free", "s256_msm_plan", "s256_hash_to_curve", "s256_expand_message_xmd",
     "s256_debug_ladder_add_count", "s256_mac32_k_dsm",
@@ -192,6 +195,20 @@ def _host(x, width):
     if width:
         a = a.reshape(-1, width)
     return a
+
+
+def ragged_rows(msgs):
+    """Messages of any length as the *_varlen entry points take them: (flat uint8 array, uint64 offsets of n + 1),
+    row i = flat[offsets[i]:offsets[i + 1]]."""
+    rows = [bytes(m) if isinstance(m, (bytes, bytearray, memoryview)) else np.ascontiguousarray(m, np.uint8).tobytes()
+            for m in msgs]
+    offsets = np.zeros(len(rows) + 1, np.uint64)
+    np.cumsum(np.fromiter((len(r) for r in rows), np.uint64, len(rows)), out=offsets[1:])
+    return np.frombuffer(b"".join(rows), np.uint8), offsets
+
+
+def _is_device_ragged(msgs):
+    return isinstance(msgs, tuple) and len(msgs) == 2 and all(_is_torch_cuda(t) for t in msgs)
 
 
 class Engine:
@@ -596,6 +613,97 @@ class Engine:
                                                 self._hp(ax), C.c_size_t(n), self._hp(sig), self._hp(st)), "schnorr_sign")
         return sig, st
 
+    # -- BIP-340 over messages of different lengths -------------------------------------------------------
+    # msgs: a sequence of bytes-like rows (host; staged by the library), or a pair of CUDA tensors (flat uint8,
+    # int64 offsets of n + 1), row i = flat[offsets[i]:offsets[i + 1]], which takes the device-resident *_dev path.
+    def _ragged_host(self, msgs, n):
+        flat, offs = ragged_rows(msgs)
+        if len(offs) != n + 1:
+            raise ValueError("length mismatch")
+        return flat, offs
+
+    def _ragged_dev(self, msgs, n):
+        import torch
+        flat, offs = msgs
+        if flat.dtype != torch.uint8 or offs.dtype != torch.int64 or not flat.is_contiguous() or not offs.is_contiguous():
+            raise S256Error("device messages must be a contiguous uint8 tensor and contiguous int64 offsets")
+        if offs.numel() != n + 1:
+            raise ValueError("length mismatch")
+        return C.c_void_p(flat.data_ptr()), C.c_void_p(offs.data_ptr())
+
+    def schnorr_verify_varlen(self, pkx32, msgs, sig64):
+        """schnorr_verify over messages of any length: ok[i] in {0, 1}."""
+        if _is_device_ragged(msgs):
+            import torch
+            n = pkx32.numel() // 32
+            if sig64.numel() != 64 * n:
+                raise ValueError("length mismatch")
+            m, o = self._ragged_dev(msgs, n)
+            ok = torch.empty(n, dtype=torch.uint8, device=pkx32.device)
+            a = self._dev_args(pkx32, sig64, ok)
+            self._check(self._lib.s256_schnorr_verify_varlen_dev(self._ctx, a[0], m, o, a[1], C.c_size_t(n), a[2],
+                                                                 self._stream()), "schnorr_verify_varlen_dev")
+            return ok
+        pk, sg = _host(pkx32, 32), _host(sig64, 64)
+        n = len(pk)
+        flat, offs = self._ragged_host(msgs, n)
+        if len(sg) != n:
+            raise ValueError("length mismatch")
+        ok = self._out(35, n)
+        self._check(self._lib.s256_schnorr_verify_varlen(self._ctx, self._hp(pk), self._hp(flat), self._hp(offs), self._hp(sg),
+                                                         C.c_size_t(n), self._hp(ok)), "schnorr_verify_varlen")
+        return ok
+
+    def schnorr_batch_verify_varlen(self, pkx32, msgs, sig64):
+        """schnorr_batch_verify over messages of any length.  With device messages: a (1,) uint8 tensor, not
+        synchronised."""
+        if _is_device_ragged(msgs):
+            import torch
+            n = pkx32.numel() // 32
+            if sig64.numel() != 64 * n:
+                raise ValueError("length mismatch")
+            m, o = self._ragged_dev(msgs, n)
+            ok = torch.empty(1, dtype=torch.uint8, device=pkx32.device)
+            a = self._dev_args(pkx32, sig64, ok)
+            self._check(self._lib.s256_schnorr_batch_verify_varlen_dev(self._ctx, a[0], m, o, a[1], C.c_size_t(n), a[2],
+                                                                       self._stream()), "schnorr_batch_verify_varlen_dev")
+            return ok
+        pk, sg = _host(pkx32, 32), _host(sig64, 64)
+        n = len(pk)
+        flat, offs = self._ragged_host(msgs, n)
+        if len(sg) != n:
+            raise ValueError("length mismatch")
+        ok = C.c_uint8(0)
+        self._check(self._lib.s256_schnorr_batch_verify_varlen(self._ctx, self._hp(pk), self._hp(flat), self._hp(offs),
+                                                               self._hp(sg), C.c_size_t(n), C.byref(ok)),
+                    "schnorr_batch_verify_varlen")
+        return bool(ok.value)
+
+    def schnorr_sign_varlen(self, priv32, msgs, aux32):
+        """schnorr_sign over messages of any length: (sig (n, 64), status (n,))."""
+        if _is_device_ragged(msgs):
+            import torch
+            n = priv32.numel() // 32
+            if aux32.numel() != 32 * n:
+                raise ValueError("length mismatch")
+            m, o = self._ragged_dev(msgs, n)
+            sig = torch.empty((n, 64), dtype=torch.uint8, device=priv32.device)
+            st = torch.empty(n, dtype=torch.uint8, device=priv32.device)
+            a = self._dev_args(priv32, aux32, sig, st)
+            self._check(self._lib.s256_schnorr_sign_varlen_dev(self._ctx, a[0], m, o, a[1], C.c_size_t(n), a[2], a[3],
+                                                               self._stream()), "schnorr_sign_varlen_dev")
+            return sig, st
+        d, ax = _host(priv32, 32), _host(aux32, 32)
+        n = len(d)
+        flat, offs = self._ragged_host(msgs, n)
+        if len(ax) != n:
+            raise ValueError("length mismatch")
+        sig = self._out(36, (n, 64))
+        st = self._out(37, n)
+        self._check(self._lib.s256_schnorr_sign_varlen(self._ctx, self._hp(d), self._hp(flat), self._hp(offs), self._hp(ax),
+                                                       C.c_size_t(n), self._hp(sig), self._hp(st)), "schnorr_sign_varlen")
+        return sig, st
+
     # -- h2c.Secp256k1_XMD_SHA256_SSWU_RO / _NU (secec/h2c/h2c.go:25,49) ------------------------
     def hash_to_curve(self, dst, msgs, random_oracle=True):
         """msgs: (n, msg_len) uint8 rows (equal length).  -> (out65, status)"""
@@ -744,6 +852,21 @@ class Engine:
                                                             self._hp(sg), C.c_size_t(n), self._hp(seed), self._hp(k),
                                                             self._hp(pts), self._hp(ssum), C.byref(rej)),
                     "debug_schnorr_batch_rows")
+        return seed.tobytes(), k, pts, ssum.tobytes(), bool(rej.value)
+
+    def debug_schnorr_batch_rows_varlen(self, pkx32, msgs, sig64):
+        """debug_schnorr_batch_rows over host messages of any length (a sequence of bytes-like rows)."""
+        pk, sg = _host(pkx32, 32), _host(sig64, 64)
+        n = len(pk)
+        flat, offs = self._ragged_host(msgs, n)
+        if n == 0 or len(sg) != n:
+            raise ValueError("length mismatch or empty batch")
+        seed, k, pts, ssum, rej = (np.zeros(32, np.uint8), np.zeros((n, 2, 32), np.uint8), np.zeros((n, 2, 64), np.uint8),
+                                   np.zeros(32, np.uint8), C.c_uint8(0))
+        self._check(self._lib.s256_debug_schnorr_batch_rows_varlen(self._ctx, self._hp(pk), self._hp(flat), self._hp(offs),
+                                                                   self._hp(sg), C.c_size_t(n), self._hp(seed), self._hp(k),
+                                                                   self._hp(pts), self._hp(ssum), C.byref(rej)),
+                    "debug_schnorr_batch_rows_varlen")
         return seed.tobytes(), k, pts, ssum.tobytes(), bool(rej.value)
 
     def debug_ecdsa_batch_rows(self, pk65, digest32, sig65, flags=0):

@@ -205,13 +205,13 @@ __global__ void __launch_bounds__(S256_TPB) k_plain_scalars(const uint8_t *u1b, 
 }
 
 // secec/bitcoin/schnorr.go:420-449: r < p, s < n (zero allowed), e = H(r||P||m) mod n;
-// R = s*G + (-e)*P (:244-245)
-__global__ void __launch_bounds__(S256_TPB) k_schnorr_scalars(const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
-                                                              const uint8_t *sig64, size_t n, sc *u1, int8_t *dig1,
-                                                              int8_t *dig2, uint8_t *sfl) {
+// R = s*G + (-e)*P (:244-245).  M: msg_uniform or msg_offsets (kernels.cuh).
+template <class M>
+__global__ void __launch_bounds__(S256_TPB) k_schnorr_scalars(const uint8_t *pkx32, M rows, const uint8_t *sig64, size_t n,
+                                                              sc *u1, int8_t *dig1, int8_t *dig2, uint8_t *sfl) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    item_schnorr_scalars(i, n, pkx32, msg, msg_len, sig64, u1, dig1, dig2, sfl);
+    item_schnorr_scalars(i, n, pkx32, rows, sig64, u1, dig1, dig2, sfl);
 }
 
 #ifndef S256_DSM_MINB
@@ -423,7 +423,7 @@ extern "C" void s256_free(s256_ctx *ctx) {
                         ctx->sink, ctx->msm_counts, ctx->msm_offsets, ctx->msm_cursor, ctx->msm_entries, ctx->msm_flag,
                         ctx->msm_buckets, ctx->msm_win, ctx->msm_acc, ctx->msm_tmp, ctx->msm_cub, ctx->msm_nsl, ctx->msm_sloff,
                         ctx->msm_perm, ctx->msm_hist, ctx->msm_range, ctx->msm_part, ctx->msm_sbkt, ctx->comm_buf, ctx->msm_aff2, ctx->msm_half, ctx->msm_bsum,
-                        ctx->bat};
+                        ctx->bat, ctx->in_off};
         for (void *p : ptrs)
             if (p) cudaFree(p);
         if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -579,11 +579,11 @@ static int chunk_ecdsa_recover(s256_ctx *ctx, const view &v, const uint8_t *dg, 
            3, pk65, status, (const uint8_t *)nullptr));
     return S256_SUCCESS;
 }
-static int chunk_schnorr_verify(s256_ctx *ctx, const view &v, const uint8_t *pkx, const uint8_t *msg, size_t msg_len,
-                                const uint8_t *sig, size_t n, uint8_t *ok, cudaStream_t s) {
+template <class M>
+static int chunk_schnorr_verify(s256_ctx *ctx, const view &v, const uint8_t *pkx, const M &rows, const uint8_t *sig, size_t n,
+                                uint8_t *ok, cudaStream_t s) {
     LAUNCH(ctx, k_decode_xonly, grid_for(n), 0, s, pkx, n, v.aff, v.pvalid);
-    LAUNCH(ctx, k_schnorr_scalars, grid_for(n), 0, s, pkx, msg, msg_len, sig, n, v.u1, v.dig1, v.dig2,
-           v.sfl);
+    LAUNCH(ctx, k_schnorr_scalars<M>, grid_for(n), 0, s, pkx, rows, sig, n, v.u1, v.dig1, v.dig2, v.sfl);
     enqueue_dsm(ctx, v, n, s);
     DISPATCH_K(n, LAUNCH(ctx, k_finish_affine<KK>, grid_for_groups(n, KK), 0, s, n, v.res, v.pvalid, v.sfl, v.cstat,
            2, (uint8_t *)nullptr, ok, sig));
@@ -803,7 +803,8 @@ extern "C" int s256_schnorr_verify_dev(s256_ctx *ctx, const uint8_t *pkx, const 
     cudaStream_t s = (cudaStream_t)stream;
     scratch_guard sg_(ctx, s, false);
     int rc = for_chunks(ctx, n, [&](size_t off, size_t c) {
-        return chunk_schnorr_verify(ctx, view_at(ctx, 0), pkx + 32 * off, msg + msg_len * off, msg_len, sig + 64 * off, c, ok + off, s);
+        return chunk_schnorr_verify(ctx, view_at(ctx, 0), pkx + 32 * off, msg_uniform{msg + msg_len * off, msg_len},
+                                    sig + 64 * off, c, ok + off, s);
     });
     return rc != S256_SUCCESS ? rc : check_launch(ctx);
 }
@@ -819,7 +820,37 @@ extern "C" int s256_schnorr_verify(s256_ctx *ctx, const uint8_t *pkx, const uint
         CK(cudaMemcpyAsync(v.in_a, pkx + 32 * off, 32 * c, cudaMemcpyHostToDevice, ps));
         if (msg_len) CK(cudaMemcpyAsync(dmsg, msg + msg_len * off, msg_len * c, cudaMemcpyHostToDevice, ps));
         CK(cudaMemcpyAsync(v.in_c, sig + 64 * off, 64 * c, cudaMemcpyHostToDevice, ps));
-        int r = chunk_schnorr_verify(ctx, v, v.in_a, dmsg, msg_len, v.in_c, c, v.st, ps);
+        int r = chunk_schnorr_verify(ctx, v, v.in_a, msg_uniform{dmsg, msg_len}, v.in_c, c, v.st, ps);
+        if (r != S256_SUCCESS) return r;
+        CK(cudaMemcpyAsync(ok + off, v.st, c, cudaMemcpyDeviceToHost, ps));
+        return S256_SUCCESS;
+    }, /*small_output=*/true);
+    return rc != S256_SUCCESS ? rc : check_launch(ctx);
+}
+extern "C" int s256_schnorr_verify_varlen_dev(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, const size_t *offsets,
+                                              const uint8_t *sig, size_t n, uint8_t *ok, void *stream) {
+    ENTER(ctx);
+    if (n && (!pkx || !msg || !offsets || !sig || !ok)) return S256_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    scratch_guard sg_(ctx, s, false);
+    int rc = for_chunks(ctx, n, [&](size_t off, size_t c) {
+        return chunk_schnorr_verify(ctx, view_at(ctx, 0), pkx + 32 * off, msg_offsets{msg, offsets + off, 0}, sig + 64 * off, c,
+                                    ok + off, s);
+    });
+    return rc != S256_SUCCESS ? rc : check_launch(ctx);
+}
+extern "C" int s256_schnorr_verify_varlen(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, const size_t *offsets,
+                                          const uint8_t *sig, size_t n, uint8_t *ok) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    if (n && (!pkx || !offsets || !sig || !ok)) return S256_ERR_ARG;
+    if (int grc = n ? varlen_staging(ctx, msg, offsets, n, ctx->cap) : S256_SUCCESS) return grc;
+    int rc = pipelined(ctx, n, [&](const view &v, size_t off, size_t c, cudaStream_t ps) {
+        msg_offsets rows;
+        CK(cudaMemcpyAsync(v.in_a, pkx + 32 * off, 32 * c, cudaMemcpyHostToDevice, ps));
+        if (int r = varlen_stage_part(ctx, msg, offsets, off, (size_t)(v.st - ctx->st), c, ps, rows)) return r;
+        CK(cudaMemcpyAsync(v.in_c, sig + 64 * off, 64 * c, cudaMemcpyHostToDevice, ps));
+        int r = chunk_schnorr_verify(ctx, v, v.in_a, rows, v.in_c, c, v.st, ps);
         if (r != S256_SUCCESS) return r;
         CK(cudaMemcpyAsync(ok + off, v.st, c, cudaMemcpyDeviceToHost, ps));
         return S256_SUCCESS;

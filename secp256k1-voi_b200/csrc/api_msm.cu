@@ -535,12 +535,17 @@ __device__ sc cta_sc_sum(sc v) {
     return sh[0];
 }
 
-__global__ void __launch_bounds__(S256_TPB) k_batch_leaves(const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
-                                                           const uint8_t *sig64, size_t n, uint32_t *leaves) {
+// M: msg_uniform or msg_offsets (kernels.cuh)
+template <class M>
+__global__ void __launch_bounds__(S256_TPB) k_batch_leaves(const uint8_t *pkx32, M rows, const uint8_t *sig64, size_t n,
+                                                           uint32_t *leaves) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     uint32_t h[8];
-    batch_leaf(h, pkx32 + 32 * i, sig64 + 64 * i, msg + msg_len * i, msg_len);
+    const uint8_t *m;
+    size_t len;
+    rows.row(i, m, len);  // an unreadable row hashes as empty; k_batch_prepare rejects it
+    batch_leaf(h, pkx32 + 32 * i, sig64 + 64 * i, m, len);
     uint4 *o = reinterpret_cast<uint4 *>(leaves + 8 * i);
     o[0] = make_uint4(h[0], h[1], h[2], h[3]);
     o[1] = make_uint4(h[4], h[5], h[6], h[7]);
@@ -597,16 +602,20 @@ __global__ void k_batch_seed(uint32_t *bat, size_t chunks, uint64_t n) {
 }
 // rows [off, off + n) of the batch -> MSM rows 2i, 2i + 1 of the chunk, part[CTA] = the CTA's sum of a_i s_i,
 // flag |= a rejected row
-__global__ void __launch_bounds__(S256_TPB) k_batch_prepare(const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
-                                                            const uint8_t *sig64, size_t n, size_t off, const uint32_t *seed_in,
-                                                            apt *aff2, uint8_t *k2, sc *part, uint32_t *flag) {
+template <class M>
+__global__ void __launch_bounds__(S256_TPB) k_batch_prepare(const uint8_t *pkx32, M rows, const uint8_t *sig64, size_t n,
+                                                            size_t off, const uint32_t *seed_in, apt *aff2, uint8_t *k2,
+                                                            sc *part, uint32_t *flag) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     sc as = sc_zero();
     if (i < n) {
         uint32_t seed[8];
         for (int k = 0; k < 8; k++) seed[k] = seed_in[k];
-        uint32_t ok = item_batch_prepare(aff2 + 2 * i, k2 + 64 * i, as, pkx32 + 32 * i, msg + msg_len * i, msg_len,
-                                         sig64 + 64 * i, seed, (uint64_t)(off + i));
+        const uint8_t *m;
+        size_t len;
+        const uint32_t row_ok = rows.row(i, m, len);
+        uint32_t ok = item_batch_prepare(aff2 + 2 * i, k2 + 64 * i, as, pkx32 + 32 * i, m, len, sig64 + 64 * i, seed,
+                                         (uint64_t)(off + i), row_ok);
         if (!ok) atomicOr(flag, 1u);
     }
     sc sum = cta_sc_sum(as);
@@ -681,22 +690,35 @@ static int batch_ensure(s256_ctx *ctx, size_t chunks) {
 // A batch's rows: three arrays of fixed-width rows (width 0: no bytes) and the flags of the call.
 //   BIP-340: a = x-only keys (32), b = messages (msg_len), c = r||s (64)
 //   ECDSA:   a = keys (65),        b = digests (32),       c = r||s||v (65)
+// BIP-340 messages of any length (the *_varlen calls) have wb = 0 and offsets: row i of b is
+// b[boff[i] - bbase, boff[i + 1] - bbase) (msg_offsets).
 struct batch_rows {
     const uint8_t *a, *b, *c;
     size_t wa, wb, wc;
     uint32_t flags;
-    batch_rows at(size_t off) const { return {a + wa * off, wb ? b + wb * off : b, c + wc * off, wa, wb, wc, flags}; }
+    const size_t *boff = nullptr;
+    size_t bbase = 0;
+    batch_rows at(size_t off) const {
+        return {a + wa * off, wb ? b + wb * off : b, c + wc * off, wa, wb, wc, flags, boff ? boff + off : boff, bbase};
+    }
 };
 // The row kinds: the seed's tag, pass 1 (leaves of c rows into `leaves`) and pass 2 (the chunk's MSM rows and per-CTA
 // G-side sums in ctx->u1; returns the number of CTA sums).
 struct batch_schnorr {
     static __host__ __device__ const char *tag() { return S256_BATCH_TAG_BIP340; }
     static void leaves(s256_ctx *ctx, const batch_rows &r, size_t c, uint32_t *leaves, cudaStream_t s) {
-        LAUNCH(ctx, k_batch_leaves, grid_for(c), 0, s, r.a, r.b, r.wb, r.c, c, leaves);
+        if (r.boff)
+            LAUNCH(ctx, k_batch_leaves<msg_offsets>, grid_for(c), 0, s, r.a, msg_offsets{r.b, r.boff, r.bbase}, r.c, c, leaves);
+        else
+            LAUNCH(ctx, k_batch_leaves<msg_uniform>, grid_for(c), 0, s, r.a, msg_uniform{r.b, r.wb}, r.c, c, leaves);
     }
     static size_t prepare(s256_ctx *ctx, const batch_rows &r, size_t c, size_t off, cudaStream_t s) {
-        LAUNCH(ctx, k_batch_prepare, grid_for(c), 0, s, r.a, r.b, r.wb, r.c, c, off, ctx->bat + BAT_SEED, ctx->aff, ctx->out,
-               ctx->u1, ctx->msm_flag);
+        if (r.boff)
+            LAUNCH(ctx, k_batch_prepare<msg_offsets>, grid_for(c), 0, s, r.a, msg_offsets{r.b, r.boff, r.bbase}, r.c, c, off,
+                   ctx->bat + BAT_SEED, ctx->aff, ctx->out, ctx->u1, ctx->msm_flag);
+        else
+            LAUNCH(ctx, k_batch_prepare<msg_uniform>, grid_for(c), 0, s, r.a, msg_uniform{r.b, r.wb}, r.c, c, off,
+                   ctx->bat + BAT_SEED, ctx->aff, ctx->out, ctx->u1, ctx->msm_flag);
         return grid_for(c);
     }
 };
@@ -788,22 +810,30 @@ static int batch_verify_dev(s256_ctx *ctx, const batch_rows &dev, size_t n, uint
     }, d_ok, s);
 }
 // The host form's rows: a batch of one chunk is copied in once and read by both passes, a longer one chunk by chunk in
-// each pass.  The verdict byte goes to ctx->st.
+// each pass.  Ragged messages go with their offsets (varlen_staging checks them first).  The verdict byte goes to ctx->st.
 template <class Kind>
 static int batch_verify_host(s256_ctx *ctx, const batch_rows &host, size_t n, const batch_chunk_fn &chunk_done = nullptr) {
     const size_t C = batch_chunk(ctx);
-    if (int grc = grow_in_b(ctx, (host.wb ? host.wb : 1) * C)) return grc;
+    if (int grc = host.boff ? varlen_staging(ctx, host.b, host.boff, n, C) : grow_in_b(ctx, (host.wb ? host.wb : 1) * C))
+        return grc;
     cudaStream_t s = ctx->stream;
     const bool resident = n <= C;
-    const batch_rows staged{ctx->in_a, ctx->in_b, ctx->in_c, host.wa, host.wb, host.wc, host.flags};
+    const batch_rows staged{ctx->in_a, ctx->in_b, ctx->in_c, host.wa, host.wb, host.wc, host.flags,
+                            host.boff ? ctx->in_off : nullptr};
     return batch_verify_run<Kind>(ctx, n, [&](size_t off, size_t c, int pass, batch_rows &r) {
         if (pass == 0 || !resident) {
             const batch_rows h = host.at(off);
             CK(cudaMemcpyAsync(ctx->in_a, h.a, h.wa * c, cudaMemcpyHostToDevice, s));
-            if (h.wb) CK(cudaMemcpyAsync(ctx->in_b, h.b, h.wb * c, cudaMemcpyHostToDevice, s));
+            msg_offsets unused;
+            if (h.boff) {
+                if (int rc = varlen_stage_part(ctx, host.b, host.boff, off, 0, c, s, unused)) return rc;
+            } else if (h.wb) {
+                CK(cudaMemcpyAsync(ctx->in_b, h.b, h.wb * c, cudaMemcpyHostToDevice, s));
+            }
             CK(cudaMemcpyAsync(ctx->in_c, h.c, h.wc * c, cudaMemcpyHostToDevice, s));
         }
         r = staged;
+        if (host.boff) r.bbase = host.boff[off];
         return S256_SUCCESS;
     }, ctx->st, s, chunk_done);
 }
@@ -878,6 +908,37 @@ extern "C" int s256_debug_schnorr_batch_rows(s256_ctx *ctx, const uint8_t *pkx, 
         return S256_ERR_ARG;
     if (ctx->cap < 2) return S256_ERR_ARG;
     return batch_debug_rows<batch_schnorr>(ctx, schnorr_rows(pkx, msg, msg_len, sig), n, seed32, k64, pts128, sum32, rejected);
+}
+
+static batch_rows schnorr_varlen_rows(const uint8_t *pkx, const uint8_t *msg, const size_t *offsets, const uint8_t *sig) {
+    return {pkx, msg, sig, 32, 0, 64, 0u, offsets};
+}
+extern "C" int s256_schnorr_batch_verify_varlen_dev(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, const size_t *offsets,
+                                                    const uint8_t *sig, size_t n, uint8_t *ok, void *stream) {
+    ENTER(ctx);
+    if (!ok || (n && (!pkx || !msg || !offsets || !sig))) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    scratch_guard sg_(ctx, s, false);
+    return batch_verify_dev<batch_schnorr>(ctx, schnorr_varlen_rows(pkx, msg, offsets, sig), n, ok, s);
+}
+extern "C" int s256_schnorr_batch_verify_varlen(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg, const size_t *offsets,
+                                                const uint8_t *sig, size_t n, uint8_t *ok) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    if (!ok || (n && (!pkx || !offsets || !sig))) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    return batch_verify_host_sync<batch_schnorr>(ctx, schnorr_varlen_rows(pkx, msg, offsets, sig), n, ok);
+}
+extern "C" int s256_debug_schnorr_batch_rows_varlen(s256_ctx *ctx, const uint8_t *pkx, const uint8_t *msg,
+                                                    const size_t *offsets, const uint8_t *sig, size_t n, uint8_t *seed32,
+                                                    uint8_t *k64, uint8_t *pts128, uint8_t *sum32, uint8_t *rejected) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    if (n == 0 || !pkx || !offsets || !sig || !seed32 || !k64 || !pts128 || !sum32 || !rejected) return S256_ERR_ARG;
+    if (ctx->cap < 2) return S256_ERR_ARG;
+    return batch_debug_rows<batch_schnorr>(ctx, schnorr_varlen_rows(pkx, msg, offsets, sig), n, seed32, k64, pts128, sum32,
+                                           rejected);
 }
 
 static batch_rows ecdsa_rows(const uint8_t *pk65, const uint8_t *digest32, const uint8_t *sig65, uint32_t flags) {

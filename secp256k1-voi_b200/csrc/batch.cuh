@@ -11,7 +11,7 @@
 // with R_i = RecoverPoint(r_i, v_i), u1_i = e_i / s_i, u2_i = r_i / s_i.  The randomizers are derived from a hash tree
 // over all the inputs, so that the batch can be hashed in parallel and in chunks:
 //
-//     leaf_i = SHA-256(pkx_i || sig_i || msg_i)              (BIP-340)
+//     leaf_i = SHA-256(pkx_i || sig_i || msg_i)              (BIP-340; msg_i of any length, >= 96 bytes hashed)
 //              SHA-256(pk65_i || digest32_i || sig65_i)      (ECDSA)
 //     node   = SHA-256(left || right); level 0 = leaves, pairs (2j, 2j + 1) upward, an unpaired last node moves up
 //              unchanged; root = the last node
@@ -153,12 +153,13 @@ S256_HD void batch_randomizer(sc &a, const uint32_t seed[8], uint64_t i) {
 // Row gi of the batch: the MSM rows -R (scalar a) and -P (scalar a e) at aff2[0..2) and k2[0..64), and as = a s for
 // the G side.  Negating the points keeps the R scalar at 128 bits, so its second endomorphism half is (almost) all
 // zero digits.  The same rejections as item_decode_xonly and item_schnorr_scalars: the key does not lift, r >= p or
-// not an x-coordinate of the curve, s >= n.  A rejected row gets G with the scalar 0 and as = 0.  Returns 1 if valid.
+// not an x-coordinate of the curve, s >= n, and a message row that cannot be read (row_ok = 0, msg_offsets).  A
+// rejected row gets G with the scalar 0 and as = 0.  Returns 1 if valid.
 S256_HD uint32_t item_batch_prepare(apt *aff2, uint8_t *k2, sc &as, const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
-                                    const uint8_t *sig64, const uint32_t seed[8], uint64_t gi) {
+                                    const uint8_t *sig64, const uint32_t seed[8], uint64_t gi, uint32_t row_ok = 1u) {
     apt P, R;
     sc s, e, a, ae;
-    uint32_t ok = item_decode_xonly(P, pkx32);
+    uint32_t ok = row_ok & item_decode_xonly(P, pkx32);
     ok &= item_decode_xonly(R, sig64);  // R = lift_x(r): r < p, and r^3 + 7 a square
     ok &= 1u - sc_from_be32(s, sig64 + 32);
     item_schnorr_challenge(e, sig64, pkx32, msg, msg_len);

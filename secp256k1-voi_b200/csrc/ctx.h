@@ -41,6 +41,8 @@ struct s256_ctx {
     // staging for the host-pointer entry points
     uint8_t *in_a = nullptr, *in_b = nullptr, *in_c = nullptr, *out = nullptr, *st = nullptr;
     size_t in_b_bytes = 0;
+    size_t *in_off = nullptr;  // the message offsets of the *_varlen host forms (allocated on first use)
+    size_t in_off_count = 0;
     unsigned long long *sink = nullptr;
     // MSM scratch (allocated on first use)
     size_t msm_cap = 0;
@@ -247,6 +249,50 @@ static inline int grow_in_b(s256_ctx *ctx, size_t need) {
     if (ctx->in_b) cudaFree(ctx->in_b);
     ctx->in_b = fresh;
     ctx->in_b_bytes = need;
+    return S256_SUCCESS;
+}
+
+// The host forms of the *_varlen entry points: message row i is msg[offsets[i], offsets[i + 1]), n + 1 offsets, and the
+// rows are staged by chunks of at most `chunk` rows.  Rejects decreasing offsets (S256_ERR_ARG, before anything is
+// enqueued) and a NULL msg under non-empty rows, then grows the staging: in_b to the bytes of the longest chunk, in_off
+// to 2 chunk + 2 offsets.  A part starting at row `so` of its chunk takes its c + 1 offsets at in_off + 2 so, so that
+// the parts of a pipelined chunk (on two streams) never write the same entry.  S256_ERR_NOMEM if that does not fit.
+static inline int varlen_staging(s256_ctx *ctx, const uint8_t *msg, const size_t *offsets, size_t n, size_t chunk) {
+    for (size_t i = 0; i < n; i++)
+        if (offsets[i + 1] < offsets[i]) return S256_ERR_ARG;
+    if (!msg && offsets[n] != offsets[0]) return S256_ERR_ARG;
+    size_t span = 1;
+    for (size_t off = 0; off < n; off += chunk) {
+        const size_t c = n - off < chunk ? n - off : chunk;
+        if (offsets[off + c] - offsets[off] > span) span = offsets[off + c] - offsets[off];
+    }
+    if (int rc = grow_in_b(ctx, span)) return rc;
+    const size_t count = 2 * (n < chunk ? n : chunk) + 2;
+    if (count <= ctx->in_off_count) return S256_SUCCESS;
+    size_t *fresh = nullptr;
+    if (cudaMalloc(&fresh, count * sizeof(size_t)) != cudaSuccess) {
+        cudaGetLastError();
+        ctx->last_err = "cudaMalloc(offset staging)";
+        return S256_ERR_NOMEM;
+    }
+    cudaStreamSynchronize(ctx->stream);
+    cudaStreamSynchronize(ctx->stream2);
+    cudaStreamSynchronize(ctx->stream3);
+    if (ctx->in_off) cudaFree(ctx->in_off);
+    ctx->in_off = fresh;
+    ctx->in_off_count = count;
+    return S256_SUCCESS;
+}
+// Stages rows [off, off + c) of a *_varlen host call whose chunk starts at row off - so: the bytes go to their place in
+// in_b (relative to the chunk's first byte), the offsets as they are to in_off + 2 so.  The rows' accessor on `s`.
+static inline int varlen_stage_part(s256_ctx *ctx, const uint8_t *msg, const size_t *offsets, size_t off, size_t so, size_t c,
+                                    cudaStream_t s, msg_offsets &rows) {
+    uint8_t *dmsg = ctx->in_b + (offsets[off] - offsets[off - so]);
+    size_t *doff = ctx->in_off + 2 * so;
+    const size_t bytes = offsets[off + c] - offsets[off];
+    if (bytes) CK(cudaMemcpyAsync(dmsg, msg + offsets[off], bytes, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(doff, offsets + off, (c + 1) * sizeof(size_t), cudaMemcpyHostToDevice, s));
+    rows = msg_offsets{dmsg, doff, offsets[off]};
     return S256_SUCCESS;
 }
 

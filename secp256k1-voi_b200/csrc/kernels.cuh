@@ -329,18 +329,55 @@ S256_HD void item_schnorr_challenge(sc &e, const uint8_t *sg, const uint8_t *pkx
     }
     sc_from_be32(e, eb);
 }
+// The message rows of the BIP-340 kernels.  row(i, p, len) points p at row i, sets its length and returns 1, or
+// returns 0 for a row that cannot be read (len = 0 then, and no byte of it is touched).  Rows are read byte by byte
+// (be32_words, sha_update), so a row may start at any address.
+//   msg_uniform: n rows of `len` bytes, row i at msg + len * i (the s256_schnorr_* entry points)
+//   msg_offsets: row i = msg[off[i] - base, off[i + 1] - base), n + 1 offsets (the *_varlen entry points).  base is
+//                the first offset of the rows the host staged at msg (0 for device rows); decreasing offsets make
+//                the row unreadable, which is how the *_varlen_dev forms reject them without a synchronisation.
+struct msg_uniform {
+    const uint8_t *msg;
+    size_t len;
+    S256_HD uint32_t row(size_t i, const uint8_t *&p, size_t &l) const {
+        p = msg + len * i;
+        l = len;
+        return 1u;
+    }
+};
+struct msg_offsets {
+    const uint8_t *msg;
+    const size_t *off;
+    size_t base;
+    S256_HD uint32_t row(size_t i, const uint8_t *&p, size_t &l) const {
+        const size_t a = off[i], b = off[i + 1];
+        const uint32_t ok = b >= a;
+        p = msg + (a - base);
+        l = ok ? b - a : 0;
+        return ok;
+    }
+};
+
 // secec/bitcoin/schnorr.go:420-449: r < p, s < n (zero allowed),
 // e = H(r||P||m) mod n; R = s*G + (-e)*P (:244-245)
-S256_HD void item_schnorr_scalars(size_t i, size_t n, const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
-                                  const uint8_t *sig64, sc *u1_out, int8_t *dig1, int8_t *dig2, uint8_t *sfl) {
+template <class M>
+S256_HD void item_schnorr_scalars(size_t i, size_t n, const uint8_t *pkx32, const M &rows, const uint8_t *sig64,
+                                  sc *u1_out, int8_t *dig1, int8_t *dig2, uint8_t *sfl) {
     const uint8_t *sg = sig64 + 64 * i;
     fe r;
     fe_from_be32(r, sg);
     sc s, e, ne;
-    uint32_t ok = fe_limbs_are_canonical(r) & (1u - sc_from_be32(s, sg + 32));
-    item_schnorr_challenge(e, sg, pkx32 + 32 * i, msg + msg_len * i, msg_len);
+    const uint8_t *m;
+    size_t len;
+    uint32_t ok = rows.row(i, m, len);
+    ok &= fe_limbs_are_canonical(r) & (1u - sc_from_be32(s, sg + 32));
+    item_schnorr_challenge(e, sg, pkx32 + 32 * i, m, len);
     sc_neg(ne, e);
     item_store_scalars(s, ne, ok, i, n, u1_out, dig1, dig2, sfl);
+}
+S256_HD void item_schnorr_scalars(size_t i, size_t n, const uint8_t *pkx32, const uint8_t *msg, size_t msg_len,
+                                  const uint8_t *sig64, sc *u1_out, int8_t *dig1, int8_t *dig2, uint8_t *sfl) {
+    item_schnorr_scalars(i, n, pkx32, msg_uniform{msg, msg_len}, sig64, u1_out, dig1, dig2, sfl);
 }
 
 // ---------------------------------------------------------------------------

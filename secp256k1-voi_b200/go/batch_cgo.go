@@ -155,6 +155,69 @@ func (e *Engine) SchnorrBatchVerify(pkx32, msgs []byte, msgLen int, sig64 []byte
 	return ok == 1, nil
 }
 
+// raggedRows flattens messages of any length into one buffer and the n + 1 offsets the *_varlen entry points take
+// (row i = flat[offsets[i]:offsets[i+1]]).  Neither holds a Go pointer, so both may be passed to C.
+func raggedRows(msgs [][]byte) (flat []byte, offsets []C.size_t) {
+	total := 0
+	for _, m := range msgs {
+		total += len(m)
+	}
+	flat = make([]byte, 0, total)
+	offsets = make([]C.size_t, len(msgs)+1)
+	for i, m := range msgs {
+		flat = append(flat, m...)
+		offsets[i+1] = C.size_t(len(flat))
+	}
+	return flat, offsets
+}
+
+// SchnorrVerifyBatchVarlen is SchnorrVerifyBatch over messages of any length, one per row.
+func (e *Engine) SchnorrVerifyBatchVarlen(pkx32 []byte, msgs [][]byte, sig64 []byte) ([]bool, error) {
+	n := len(msgs)
+	if len(pkx32) != 32*n || len(sig64) != 64*n {
+		panic("secp256k1b200: SchnorrVerifyBatchVarlen: length mismatch")
+	}
+	flat, offs := raggedRows(msgs)
+	ok := make([]byte, n)
+	if err := e.err(C.s256_schnorr_verify_varlen(e.ctx, ptr(pkx32), ptr(flat), &offs[0], ptr(sig64), C.size_t(n), ptr(ok))); err != nil {
+		return nil, err
+	}
+	out := make([]bool, n)
+	for i, v := range ok {
+		out[i] = v == 1
+	}
+	return out, nil
+}
+
+// SchnorrBatchVerifyVarlen is SchnorrBatchVerify over messages of any length, one per row.
+func (e *Engine) SchnorrBatchVerifyVarlen(pkx32 []byte, msgs [][]byte, sig64 []byte) (bool, error) {
+	n := len(msgs)
+	if len(pkx32) != 32*n || len(sig64) != 64*n {
+		panic("secp256k1b200: SchnorrBatchVerifyVarlen: length mismatch")
+	}
+	flat, offs := raggedRows(msgs)
+	var ok C.uint8_t
+	if err := e.err(C.s256_schnorr_batch_verify_varlen(e.ctx, ptr(pkx32), ptr(flat), &offs[0], ptr(sig64), C.size_t(n), &ok)); err != nil {
+		return false, err
+	}
+	return ok == 1, nil
+}
+
+// SchnorrSignBatchVarlen is bitcoin.SchnorrPrivateKey.Sign over rows of priv32 (d'), one message of any length and
+// 32 bytes of auxiliary randomness each: sig64 and a status byte per row (S256_ST_OK / S256_ST_INVALID).
+func (e *Engine) SchnorrSignBatchVarlen(priv32 []byte, msgs [][]byte, aux32 []byte) (sig64, status []byte, err error) {
+	n := len(msgs)
+	if len(priv32) != 32*n || len(aux32) != 32*n {
+		panic("secp256k1b200: SchnorrSignBatchVarlen: length mismatch")
+	}
+	flat, offs := raggedRows(msgs)
+	sig64, status = make([]byte, 64*n), make([]byte, n)
+	if err := e.err(C.s256_schnorr_sign_varlen(e.ctx, ptr(priv32), ptr(flat), &offs[0], ptr(aux32), C.size_t(n), ptr(sig64), ptr(status))); err != nil {
+		return nil, nil, err
+	}
+	return sig64, status, nil
+}
+
 // ScalarBaseMultBatch is Point.ScalarBaseMult + UncompressedBytes (constant time).
 func (e *Engine) ScalarBaseMultBatch(scalars []*secp256k1.Scalar) ([]*secp256k1.Point, error) {
 	n := len(scalars)

@@ -866,6 +866,42 @@ inline bool SchnorrBatchVerify(const uint8_t *pkx32, const uint8_t *msg, size_t 
     e.check(s256_schnorr_batch_verify(e.ctx(), pkx32, msg, msg_len, sig64, n, &ok), "SchnorrBatchVerify");
     return ok == 1;
 }
+// The same over messages of any length, one per row (msgs.size() rows): flattened with n + 1 offsets for the
+// *_varlen entry points.
+namespace detail {
+struct RaggedRows {
+    std::vector<uint8_t> flat;
+    std::vector<size_t> offsets{0};
+    explicit RaggedRows(const std::vector<std::vector<uint8_t>> &msgs) {
+        for (const auto &m : msgs) {
+            flat.insert(flat.end(), m.begin(), m.end());
+            offsets.push_back(flat.size());
+        }
+    }
+    const uint8_t *data() const { return flat.empty() ? nullptr : flat.data(); }
+};
+}  // namespace detail
+inline void SchnorrVerifyBatch(const uint8_t *pkx32, const std::vector<std::vector<uint8_t>> &msgs, const uint8_t *sig64,
+                               uint8_t *ok, Engine &e = Engine::Default()) {
+    detail::RaggedRows r(msgs);
+    e.check(s256_schnorr_verify_varlen(e.ctx(), pkx32, r.data(), r.offsets.data(), sig64, msgs.size(), ok), "SchnorrVerifyBatch");
+}
+inline bool SchnorrBatchVerify(const uint8_t *pkx32, const std::vector<std::vector<uint8_t>> &msgs, const uint8_t *sig64,
+                               Engine &e = Engine::Default()) {
+    detail::RaggedRows r(msgs);
+    uint8_t ok = 0;
+    e.check(s256_schnorr_batch_verify_varlen(e.ctx(), pkx32, r.data(), r.offsets.data(), sig64, msgs.size(), &ok),
+            "SchnorrBatchVerify");
+    return ok == 1;
+}
+// SchnorrPrivateKey.Sign over rows: priv32 (d' as for NewSchnorrPrivateKey), one message of any length and 32 bytes
+// of auxiliary randomness per row -> sig64 and a status byte per row (S256_ST_OK or S256_ST_INVALID).
+inline void SchnorrSignBatch(const uint8_t *priv32, const std::vector<std::vector<uint8_t>> &msgs, const uint8_t *aux32,
+                             uint8_t *sig64, uint8_t *status, Engine &e = Engine::Default()) {
+    detail::RaggedRows r(msgs);
+    e.check(s256_schnorr_sign_varlen(e.ctx(), priv32, r.data(), r.offsets.data(), aux32, msgs.size(), sig64, status),
+            "SchnorrSignBatch");
+}
 }  // namespace bitcoin
 
 namespace h2c {
