@@ -130,9 +130,11 @@ int s256_ecdsa_verify_dev(s256_ctx *ctx, const uint8_t *d_pk65, const uint8_t *d
  *     SEQUENCE{r,s}, both in [1, n) -> r||s rows; ok[i] = 0 (row zeroed) when rejected.
  *   s256_is_valid_signature_encoding_bip0066: bitcoin.IsValidSignatureEncodingBIP0066
  *     (secec/bitcoin/asn1_shitcoin.go:13), rows INCLUDE the trailing sighash byte.
- *   s256_ecdsa_verify_asn1: PublicKey.Verify with EncodingASN1 (secec/ecdsa.go:171-228).
+ *   s256_ecdsa_verify_asn1: PublicKey.Verify with EncodingASN1 (secec/ecdsa.go:171-228).  The rows are
+ *     staged to the device and parsed there (the parse of s256_parse_asn1_signatures); S256_ERR_ARG for
+ *     decreasing offsets, checked before anything is enqueued.
  *   s256_bitcoin_verify_asn1: bitcoin.VerifyASN1 (secec/bitcoin/ecdsa_shitcoin.go:29): BIP-66
- *     check, sighash byte stripped, s <= n/2 enforced.
+ *     check, sighash byte stripped, s <= n/2 enforced; parsed on the device as above.
  *   s256_parse_asn1_public_keys: secec.ParseASN1PublicKey (secec/s11n.go:38-76) up to the call of
  *     NewPublicKey: strict SubjectPublicKeyInfo with the ecPublicKey / secp256k1 OIDs; yields the
  *     SEC 1 point bytes (row stride 65, left-aligned, point_len[i] in {1, 33, 65}) and a status
@@ -159,6 +161,25 @@ int s256_ecdsa_verify_asn1(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *di
                            const size_t *offsets, uint32_t flags, size_t n, uint8_t *ok);
 int s256_bitcoin_verify_asn1(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32, const uint8_t *der,
                              const size_t *offsets, size_t n, uint8_t *ok);
+/* Device-resident DER signatures.  d_der and d_offsets live in device memory: d_offsets holds n + 1 values relative
+ * to d_der (offsets[0] need not be 0), row i being d_der[offsets[i] .. offsets[i+1]).  These forms cannot check the
+ * offsets without synchronising, so a row with offsets[i+1] < offsets[i] is invalid and none of its bytes are read
+ * (ok[i] = 0, and a zeroed r||s row).  The host forms of all four return S256_ERR_ARG for such offsets instead.  One
+ * thread parses one row and reads at most 73 bytes of it: a row longer than that is rejected from its length alone
+ * (no strict-DER signature exceeds 72 bytes, and BIP-66 allows at most 73 with the sighash byte), in the host forms
+ * too.  No form synchronises; outputs are written on `stream`.
+ *   s256_ecdsa_verify_asn1_dev: s256_ecdsa_verify_asn1 (flags as for s256_ecdsa_verify).
+ *   s256_bitcoin_verify_asn1_dev: s256_bitcoin_verify_asn1; S256_FLAG_REJECT_MALLEABLE is implied.
+ *   s256_parse_asn1_signatures_dev: the sig64 and ok bytes of s256_parse_asn1_signatures.
+ *   s256_is_valid_signature_encoding_bip0066_dev: the ok bytes of s256_is_valid_signature_encoding_bip0066. */
+int s256_ecdsa_verify_asn1_dev(s256_ctx *ctx, const uint8_t *d_pk65, const uint8_t *d_digest32, const uint8_t *d_der,
+                               const size_t *d_offsets, uint32_t flags, size_t n, uint8_t *d_ok, void *stream);
+int s256_bitcoin_verify_asn1_dev(s256_ctx *ctx, const uint8_t *d_pk65, const uint8_t *d_digest32, const uint8_t *d_der,
+                                 const size_t *d_offsets, size_t n, uint8_t *d_ok, void *stream);
+int s256_parse_asn1_signatures_dev(s256_ctx *ctx, const uint8_t *d_der, const size_t *d_offsets, size_t n, uint8_t *d_sig64,
+                                   uint8_t *d_ok, void *stream);
+int s256_is_valid_signature_encoding_bip0066_dev(s256_ctx *ctx, const uint8_t *d_der, const size_t *d_offsets, size_t n,
+                                                 uint8_t *d_ok, void *stream);
 
 /* --- PrivateKey.Sign with RFC6979SHA256() as the entropy source (secec/ecdsa.go:92-135,284-390;
  *     nonce: secec/ecdsa_k_rfc6979.go): deterministic, constant time.  priv32 must be a canonical

@@ -27,6 +27,9 @@ for n in (1, 33, 1500):
     eng.schnorr_sign(priv, w["digest32"], ks)
     eng.hash_to_curve(b"QUUX-V01-CS02-with-secp256k1_XMD:SHA-256_SSWU_RO_", w["digest32"], random_oracle=True)
     eng.new_public_keys([bytes(r) for r in pk[:8]] + [b"\x00", b"\x02" + bytes(pk[-1][1:33])])
+    der = pkg.build_asn1_signatures(w["sig64"])
+    eng.ecdsa_verify_asn1(w["pk65"], w["digest32"], der)
+    eng.bitcoin_verify_asn1(w["pk65"], w["digest32"], [r + b"\x01" for r in der])
 # the sort / slice / super-slice / window stages of the MSM: random scalars, then one heavy bucket per window
 wm = pkg.synth.msm_batch(6000, eng.scalar_base_mult)
 eng.msm(wm["k32"], wm["pt65"])
@@ -47,6 +50,17 @@ with torch.cuda.stream(s2):
     b = eng.ecdsa_verify(*d)
 torch.cuda.synchronize()
 assert np.array_equal(a.cpu().numpy(), w["expected"]) and np.array_equal(b.cpu().numpy(), w["expected"])
+# the device-resident DER entry points (misaligned rows: the parse reads byte by byte)
+for rows in (pkg.build_asn1_signatures(w["sig64"]), [r + b"\x01" for r in pkg.build_asn1_signatures(w["sig64"])]):
+    flat, offs = pkg.ragged_rows(rows)
+    dflat = torch.zeros(len(flat) + 1, dtype=torch.uint8, device="cuda")
+    dflat[1:] = torch.from_numpy(flat.copy()).cuda()
+    dd = (dflat, torch.from_numpy(offs.astype(np.int64) + 1).cuda())
+    eng.ecdsa_verify_asn1(d[0], d[1], dd)
+    eng.bitcoin_verify_asn1(d[0], d[1], dd)
+    eng.parse_asn1_signatures_dev(dd)
+    eng.is_valid_signature_encoding_bip0066_dev(dd)
+torch.cuda.synchronize()
 eng.close()
 mid = pkg.Engine(device=0, max_batch=1 << 16)
 wmid = pkg.synth.msm_batch(1 << 16, mid.scalar_base_mult)

@@ -35,7 +35,8 @@ EXPORTED_SYMBOLS = [
     "s256_parse_asn1_signatures", "s256_is_valid_signature_encoding_bip0066",
     "s256_parse_asn1_public_keys", "s256_build_asn1_public_keys", "s256_build_asn1_signatures",
     "s256_new_public_keys", "s256_parse_asn1_public_keys_checked",
-    "s256_ecdsa_verify_asn1", "s256_bitcoin_verify_asn1",
+    "s256_ecdsa_verify_asn1", "s256_bitcoin_verify_asn1", "s256_ecdsa_verify_asn1_dev", "s256_bitcoin_verify_asn1_dev",
+    "s256_parse_asn1_signatures_dev", "s256_is_valid_signature_encoding_bip0066_dev",
     "s256_ecdsa_recover", "s256_ecdsa_recover_dev",
     "s256_ecdsa_recoverable_batch_verify", "s256_ecdsa_recoverable_batch_verify_dev",
     "s256_ecdsa_sign_rfc6979", "s256_ecdsa_sign_rfc6979_dev",
@@ -449,7 +450,21 @@ class Engine:
         return ok
 
     # -- PublicKey.Verify, EncodingASN1 (secec/ecdsa.go:171) and bitcoin.VerifyASN1 ----------
+    # der_rows: a sequence of bytes-like rows (host), or a pair of CUDA tensors (flat uint8, int64 offsets of n + 1),
+    # row i = flat[offsets[i]:offsets[i + 1]], which takes the device-resident *_dev path (pk65 and digest32 are then
+    # CUDA tensors too, and the ok tensor is returned without synchronising).
     def ecdsa_verify_asn1(self, pk65, digest32, der_rows, flags=0):
+        if _is_device_ragged(der_rows):
+            import torch
+            n = pk65.numel() // 65
+            if digest32.numel() != 32 * n:
+                raise ValueError("length mismatch")
+            d, o = self._ragged_dev(der_rows, n)
+            ok = torch.empty(n, dtype=torch.uint8, device=pk65.device)
+            a = self._dev_args(pk65, digest32, ok)
+            self._check(self._lib.s256_ecdsa_verify_asn1_dev(self._ctx, a[0], a[1], d, o, C.c_uint32(flags), C.c_size_t(n),
+                                                             a[2], self._stream()), "ecdsa_verify_asn1_dev")
+            return ok
         pk, dg = _host(pk65, 65), _host(digest32, 32)
         data, offs = _pack_rows(der_rows)
         n = len(der_rows)
@@ -461,6 +476,17 @@ class Engine:
         return ok
 
     def bitcoin_verify_asn1(self, pk65, digest32, der_rows_with_sighash):
+        if _is_device_ragged(der_rows_with_sighash):
+            import torch
+            n = pk65.numel() // 65
+            if digest32.numel() != 32 * n:
+                raise ValueError("length mismatch")
+            d, o = self._ragged_dev(der_rows_with_sighash, n)
+            ok = torch.empty(n, dtype=torch.uint8, device=pk65.device)
+            a = self._dev_args(pk65, digest32, ok)
+            self._check(self._lib.s256_bitcoin_verify_asn1_dev(self._ctx, a[0], a[1], d, o, C.c_size_t(n), a[2],
+                                                               self._stream()), "bitcoin_verify_asn1_dev")
+            return ok
         pk, dg = _host(pk65, 65), _host(digest32, 32)
         data, offs = _pack_rows(der_rows_with_sighash)
         n = len(der_rows_with_sighash)
@@ -469,6 +495,32 @@ class Engine:
         ok = self._out(18, n)
         self._check(self._lib.s256_bitcoin_verify_asn1(self._ctx, self._hp(pk), self._hp(dg), self._hp(data), self._hp(offs),
                                                        C.c_size_t(n), self._hp(ok)), "bitcoin_verify_asn1")
+        return ok
+
+    def parse_asn1_signatures_dev(self, der_rows):
+        """parse_asn1_signatures on the device: der_rows is a (flat uint8, int64 offsets) pair of CUDA tensors.
+        -> (sig64 (n, 64), ok (n,)) CUDA tensors, not synchronised."""
+        import torch
+        n = der_rows[1].numel() - 1
+        d, o = self._ragged_dev(der_rows, n)
+        sig = torch.empty((n, 64), dtype=torch.uint8, device=der_rows[0].device)
+        ok = torch.empty(n, dtype=torch.uint8, device=der_rows[0].device)
+        a = self._dev_args(sig, ok)
+        self._check(self._lib.s256_parse_asn1_signatures_dev(self._ctx, d, o, C.c_size_t(n), a[0], a[1], self._stream()),
+                    "parse_asn1_signatures_dev")
+        return sig, ok
+
+    def is_valid_signature_encoding_bip0066_dev(self, der_rows_with_sighash):
+        """is_valid_signature_encoding_bip0066 on the device: a (flat uint8, int64 offsets) pair of CUDA tensors.
+        -> ok (n,) CUDA tensor, not synchronised."""
+        import torch
+        n = der_rows_with_sighash[1].numel() - 1
+        d, o = self._ragged_dev(der_rows_with_sighash, n)
+        ok = torch.empty(n, dtype=torch.uint8, device=der_rows_with_sighash[0].device)
+        a = self._dev_args(ok)
+        self._check(self._lib.s256_is_valid_signature_encoding_bip0066_dev(self._ctx, d, o, C.c_size_t(n), a[0],
+                                                                           self._stream()),
+                    "is_valid_signature_encoding_bip0066_dev")
         return ok
 
     # -- PrivateKey.Sign(RFC6979SHA256(), digest) (secec/ecdsa.go:92,284) -------------------

@@ -5,6 +5,7 @@
 // CPU implementation of any curve operation in this library: without a CUDA
 // device every entry point fails with S256_ERR_NO_DEVICE.
 #include "ctx.h"
+#include "der.cuh"
 #include "microbench.cuh"
 
 // ---------------------------------------------------------------------------
@@ -212,6 +213,24 @@ __global__ void __launch_bounds__(S256_TPB) k_schnorr_scalars(const uint8_t *pkx
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     item_schnorr_scalars(i, n, pkx32, rows, sig64, u1, dig1, dig2, sfl);
+}
+
+// Strict-DER (BIP66 = false) or BIP-66 + strict-DER rows (der.cuh) -> r||s rows, zeros where rejected, and one ok
+// byte per row; either output may be NULL.  M: msg_offsets.
+template <class M, bool BIP66>
+__global__ void __launch_bounds__(S256_TPB) k_parse_der(M rows, size_t n, uint8_t *sig64, uint8_t *ok) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint32_t rs[16];
+    const uint32_t good = item_parse_der<BIP66>(i, rows, rs);
+    if (sig64) der_store_sig64(sig64 + 64 * i, rs);
+    if (ok) ok[i] = (uint8_t)good;
+}
+template <class M>
+__global__ void __launch_bounds__(S256_TPB) k_check_bip66(M rows, size_t n, uint8_t *ok) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    ok[i] = (uint8_t)item_check_bip66(i, rows);
 }
 
 #ifndef S256_DSM_MINB
@@ -1043,50 +1062,108 @@ extern "C" int s256_parse_asn1_public_keys_checked(s256_ctx *ctx, const uint8_t 
     }
 }
 
-// PublicKey.Verify with EncodingASN1 (secec/ecdsa.go:171-228): parse on the host (codecs.cpp), then the
-// same batch as the compact path; rows the parser rejects come back false.
+// PublicKey.Verify with EncodingASN1 (secec/ecdsa.go:171-228) and bitcoin.VerifyASN1 (secec/bitcoin/ecdsa_shitcoin.go:29-35):
+// k_parse_der writes the chunk's r||s rows to in_c, all zero for a row it rejects, and the compact verification runs
+// on them.  r = 0 fails k_ecdsa_scalars' range check, so a rejected row comes back false without a separate AND.
+template <bool BIP66>
+static int chunk_der_verify(s256_ctx *ctx, const view &v, const uint8_t *pk, const uint8_t *dg, const msg_offsets &rows,
+                            uint32_t flags, size_t n, uint8_t *ok, cudaStream_t s) {
+    LAUNCH(ctx, (k_parse_der<msg_offsets, BIP66>), grid_for(n), 0, s, rows, n, v.in_c, (uint8_t *)nullptr);
+    return chunk_ecdsa_verify(ctx, v, pk, dg, v.in_c, flags, n, ok, s);
+}
+template <bool BIP66>
+static int der_verify_dev(s256_ctx *ctx, const uint8_t *pk, const uint8_t *dg, const uint8_t *der, const size_t *offsets,
+                          uint32_t flags, size_t n, uint8_t *ok, void *stream) {
+    ENTER(ctx);
+    if (n && (!pk || !dg || !der || !offsets || !ok)) return S256_ERR_ARG;
+    cudaStream_t s = (cudaStream_t)stream;
+    scratch_guard sg_(ctx, s, false);
+    int rc = for_chunks(ctx, n, [&](size_t off, size_t c) {
+        return chunk_der_verify<BIP66>(ctx, view_at(ctx, 0), pk + 65 * off, dg + 32 * off, msg_offsets{der, offsets + off, 0},
+                                       flags, c, ok + off, s);
+    });
+    return rc != S256_SUCCESS ? rc : check_launch(ctx);
+}
+// The host forms stage the DER rows as the *_varlen host forms stage messages (in_b, in_off), so the digests go to
+// `out`.  A row longer than DER_ROW_MAX is rejected from its length alone, so its bytes are never staged: when there is
+// such a row, the rows are staged from a compacted copy in which it is empty (an empty row is rejected too).
+template <bool BIP66>
+static int der_verify_host(s256_ctx *ctx, const uint8_t *pk, const uint8_t *dg, const uint8_t *der, const size_t *offsets,
+                           uint32_t flags, size_t n, uint8_t *ok) {
+    ENTER(ctx);
+    scratch_guard sg_(ctx, ctx->stream, true);
+    bool long_rows = false;
+    for (size_t i = 0; i < n; i++) {
+        if (offsets[i + 1] < offsets[i]) return S256_ERR_ARG;
+        long_rows |= offsets[i + 1] - offsets[i] > DER_ROW_MAX;
+    }
+    std::vector<uint8_t> short_bytes;
+    std::vector<size_t> short_offsets;
+    if (long_rows) {
+        try {
+            short_offsets.resize(n + 1);
+            for (size_t i = 0; i < n; i++) {
+                short_offsets[i] = short_bytes.size();
+                if (offsets[i + 1] - offsets[i] <= DER_ROW_MAX)
+                    short_bytes.insert(short_bytes.end(), der + offsets[i], der + offsets[i + 1]);
+            }
+            short_offsets[n] = short_bytes.size();
+        } catch (const std::bad_alloc &) {
+            return S256_ERR_NOMEM;
+        }
+        der = short_bytes.data();
+        offsets = short_offsets.data();
+    }
+    if (int grc = varlen_staging(ctx, der, offsets, n, ctx->cap)) return grc;
+    int rc = pipelined(ctx, n, [&](const view &v, size_t off, size_t c, cudaStream_t ps) {
+        msg_offsets rows;
+        CK(cudaMemcpyAsync(v.out, dg + 32 * off, 32 * c, cudaMemcpyHostToDevice, ps));
+        if (int r = varlen_stage_part(ctx, der, offsets, off, (size_t)(v.st - ctx->st), c, ps, rows)) return r;
+        CK(cudaMemcpyAsync(v.in_a, pk + 65 * off, 65 * c, cudaMemcpyHostToDevice, ps));
+        int r = chunk_der_verify<BIP66>(ctx, v, v.in_a, v.out, rows, flags, c, v.st, ps);
+        if (r != S256_SUCCESS) return r;
+        CK(cudaMemcpyAsync(ok + off, v.st, c, cudaMemcpyDeviceToHost, ps));
+        return S256_SUCCESS;
+    }, /*small_output=*/true);
+    return rc != S256_SUCCESS ? rc : check_launch(ctx);
+}
 extern "C" int s256_ecdsa_verify_asn1(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32, const uint8_t *der,
                                       const size_t *offsets, uint32_t flags, size_t n, uint8_t *ok) {
     if (!ctx || (n && (!pk65 || !digest32 || !der || !offsets || !ok))) return S256_ERR_ARG;
     if (n == 0) return S256_SUCCESS;
-    try {
-        std::vector<uint8_t> sig(64 * n), parsed(n);
-        int rc = s256_parse_asn1_signatures(der, offsets, n, sig.data(), parsed.data());
-        if (rc != S256_SUCCESS) return rc;
-        rc = s256_ecdsa_verify(ctx, pk65, digest32, sig.data(), flags, n, ok);
-        if (rc != S256_SUCCESS) return rc;
-        for (size_t i = 0; i < n; i++) ok[i] &= parsed[i];
-        return S256_SUCCESS;
-    } catch (const std::bad_alloc &) {
-        return S256_ERR_NOMEM;
-    }
+    return der_verify_host<false>(ctx, pk65, digest32, der, offsets, flags, n, ok);
 }
-// bitcoin.VerifyASN1 (secec/bitcoin/ecdsa_shitcoin.go:29-35)
+extern "C" int s256_ecdsa_verify_asn1_dev(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32, const uint8_t *der,
+                                          const size_t *offsets, uint32_t flags, size_t n, uint8_t *ok, void *stream) {
+    return der_verify_dev<false>(ctx, pk65, digest32, der, offsets, flags, n, ok, stream);
+}
+// bitcoin.VerifyASN1: rows carry the sighash byte; s <= n/2 is enforced
 extern "C" int s256_bitcoin_verify_asn1(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32, const uint8_t *der,
                                         const size_t *offsets, size_t n, uint8_t *ok) {
     if (!ctx || (n && (!pk65 || !digest32 || !der || !offsets || !ok))) return S256_ERR_ARG;
     if (n == 0) return S256_SUCCESS;  // (offsets may be NULL then)
-    try {
-        std::vector<uint8_t> bip(n);
-        int rc = s256_is_valid_signature_encoding_bip0066(der, offsets, n, bip.data());
-        if (rc != S256_SUCCESS) return rc;
-        // strip the sighash byte of the rows that passed; rejected rows become empty (and fail to parse)
-        std::vector<size_t> off2(n + 1);
-        std::vector<uint8_t> der2;
-        der2.reserve(offsets[n] - offsets[0]);
-        for (size_t i = 0; i < n; i++) {
-            off2[i] = der2.size();
-            if (bip[i]) der2.insert(der2.end(), der + offsets[i], der + offsets[i + 1] - 1);
-        }
-        off2[n] = der2.size();
-        if (der2.empty()) der2.push_back(0);
-        rc = s256_ecdsa_verify_asn1(ctx, pk65, digest32, der2.data(), off2.data(), S256_FLAG_REJECT_MALLEABLE, n, ok);
-        if (rc != S256_SUCCESS) return rc;
-        for (size_t i = 0; i < n; i++) ok[i] &= bip[i];
-        return S256_SUCCESS;
-    } catch (const std::bad_alloc &) {
-        return S256_ERR_NOMEM;
-    }
+    return der_verify_host<true>(ctx, pk65, digest32, der, offsets, S256_FLAG_REJECT_MALLEABLE, n, ok);
+}
+extern "C" int s256_bitcoin_verify_asn1_dev(s256_ctx *ctx, const uint8_t *pk65, const uint8_t *digest32, const uint8_t *der,
+                                            const size_t *offsets, size_t n, uint8_t *ok, void *stream) {
+    return der_verify_dev<true>(ctx, pk65, digest32, der, offsets, S256_FLAG_REJECT_MALLEABLE, n, ok, stream);
+}
+// The device twins of the host codecs s256_parse_asn1_signatures and s256_is_valid_signature_encoding_bip0066.  They use
+// no context scratch, so they need no scratch_guard.
+extern "C" int s256_parse_asn1_signatures_dev(s256_ctx *ctx, const uint8_t *der, const size_t *offsets, size_t n,
+                                              uint8_t *sig64, uint8_t *ok, void *stream) {
+    ENTER(ctx);
+    if (n && (!der || !offsets || !sig64 || !ok)) return S256_ERR_ARG;
+    if (n) LAUNCH(ctx, (k_parse_der<msg_offsets, false>), grid_for(n), 0, (cudaStream_t)stream, msg_offsets{der, offsets, 0}, n,
+                  sig64, ok);
+    return check_launch(ctx);
+}
+extern "C" int s256_is_valid_signature_encoding_bip0066_dev(s256_ctx *ctx, const uint8_t *der, const size_t *offsets, size_t n,
+                                                            uint8_t *ok, void *stream) {
+    ENTER(ctx);
+    if (n && (!der || !offsets || !ok)) return S256_ERR_ARG;
+    if (n) LAUNCH(ctx, k_check_bip66<msg_offsets>, grid_for(n), 0, (cudaStream_t)stream, msg_offsets{der, offsets, 0}, n, ok);
+    return check_launch(ctx);
 }
 
 // ---------------------------------------------------------------------------
