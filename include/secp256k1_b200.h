@@ -290,6 +290,28 @@ int s256_hash_to_curve(s256_ctx *ctx, const uint8_t *dst, size_t dst_len, const 
                        int random_oracle, uint8_t *out65, uint8_t *status);
 int s256_expand_message_xmd(s256_ctx *ctx, const uint8_t *dst, size_t dst_len, const uint8_t *msg, size_t msg_len,
                             size_t n, size_t len_in_bytes, uint8_t *out);
+/* The same over device-resident rows, and over messages of different lengths.  Row i's out65 and status are those of
+ * s256_hash_to_curve on that row alone.  The DST stays a host pointer in every form (one public parameter per call,
+ * with the rules above); the _dev forms pass it to the device inside a kernel launch, so they read no host memory of
+ * the caller after returning.
+ *   s256_hash_to_curve_dev: d_msg, d_out65 and d_status are device pointers (any alignment).
+ *   s256_hash_to_curve_varlen: messages concatenated in `msg` as for s256_schnorr_verify_varlen: row i is
+ *     msg[offsets[i] .. offsets[i+1]), n + 1 offsets (offsets[0] need not be 0); msg may be NULL when every row is
+ *     empty.  S256_ERR_ARG for decreasing offsets, checked before anything is enqueued; S256_ERR_NOMEM when the
+ *     message bytes of one chunk (max_batch rows) do not fit the device staging.
+ *   s256_hash_to_curve_varlen_dev: d_offsets is a device array of n + 1 values relative to d_msg.  This form cannot
+ *     check it without synchronising, so a row with offsets[i+1] < offsets[i] reads none of its bytes and gets
+ *     S256_ST_INVALID with 65 zero bytes (a status the uniform forms never return).
+ * The _dev forms do not synchronise; outputs are written on `stream`.  Hashing is constant time in the message bytes
+ * and the DST, not in the message length (as in the reference, whose SHA-256 also runs longer on longer input): one
+ * thread hashes one row, so a warp waits for its longest message and a very long message slows the 31 rows beside it. */
+int s256_hash_to_curve_dev(s256_ctx *ctx, const uint8_t *dst, size_t dst_len, const uint8_t *d_msg, size_t msg_len,
+                           size_t n, int random_oracle, uint8_t *d_out65, uint8_t *d_status, void *stream);
+int s256_hash_to_curve_varlen(s256_ctx *ctx, const uint8_t *dst, size_t dst_len, const uint8_t *msg,
+                              const size_t *offsets, size_t n, int random_oracle, uint8_t *out65, uint8_t *status);
+int s256_hash_to_curve_varlen_dev(s256_ctx *ctx, const uint8_t *dst, size_t dst_len, const uint8_t *d_msg,
+                                  const size_t *d_offsets, size_t n, int random_oracle, uint8_t *d_out65,
+                                  uint8_t *d_status, void *stream);
 
 /* --- Point.MultiScalarMult[Vartime] (point_mul_multi.go:25,73): sum k_i*P_i
  *     over this context's items -> one 65-byte point.  n == 0 gives the

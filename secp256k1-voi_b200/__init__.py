@@ -47,6 +47,7 @@ EXPORTED_SYMBOLS = [
     "s256_debug_schnorr_batch_rows_varlen",
     "s256_msm", "s256_msm_partial", "s256_msm_combine", "s256_msm_dev", "s256_msm_sharded", "s256_msm_sharded_dev",
     "s256_comm_unique_id", "s256_comm_init", "s256_comm_free", "s256_msm_plan", "s256_hash_to_curve", "s256_expand_message_xmd",
+    "s256_hash_to_curve_dev", "s256_hash_to_curve_varlen", "s256_hash_to_curve_varlen_dev",
     "s256_debug_ladder_add_count", "s256_mac32_k_dsm",
     "s256_debug_gen_table", "s256_debug_field_op", "s256_debug_schnorr_batch_rows", "s256_debug_ecdsa_batch_rows",
     "s256_microbench_imad",
@@ -758,8 +759,21 @@ class Engine:
 
     # -- h2c.Secp256k1_XMD_SHA256_SSWU_RO / _NU (secec/h2c/h2c.go:25,49) ------------------------
     def hash_to_curve(self, dst, msgs, random_oracle=True):
-        """msgs: (n, msg_len) uint8 rows (equal length).  -> (out65, status)"""
+        """msgs: (n, msg_len) uint8 rows (equal length), host or CUDA.  -> (out65, status); with a CUDA tensor the
+        device-resident _dev path runs and the results are CUDA tensors, not synchronised."""
         dst = bytes(dst)
+        if _is_torch_cuda(msgs):
+            import torch
+            if msgs.dim() != 2:
+                raise ValueError("msgs must be a 2-D tensor of equal-length rows")
+            n, msg_len = msgs.shape
+            out = torch.empty((n, 65), dtype=torch.uint8, device=msgs.device)
+            st = torch.empty(n, dtype=torch.uint8, device=msgs.device)
+            a = self._dev_args(msgs, out, st)
+            self._check(self._lib.s256_hash_to_curve_dev(self._ctx, dst, C.c_size_t(len(dst)), a[0], C.c_size_t(msg_len),
+                                                         C.c_size_t(n), int(bool(random_oracle)), a[1], a[2], self._stream()),
+                        "hash_to_curve_dev")
+            return out, st
         m = np.ascontiguousarray(msgs, dtype=np.uint8)
         if m.ndim != 2:
             raise ValueError("msgs must be a 2-D array of equal-length rows")
@@ -769,6 +783,31 @@ class Engine:
         self._check(self._lib.s256_hash_to_curve(self._ctx, dst, C.c_size_t(len(dst)), self._hp(m), C.c_size_t(msg_len),
                                                  C.c_size_t(n), int(bool(random_oracle)), self._hp(out), self._hp(st)),
                     "hash_to_curve")
+        return out, st
+
+    def hash_to_curve_varlen(self, dst, msgs, random_oracle=True):
+        """hash_to_curve over messages of any length: a sequence of bytes-like rows, or a (flat uint8, int64 offsets)
+        pair of CUDA tensors (the _dev path: CUDA results, not synchronised).  -> (out65 (n, 65), status (n,)); a
+        device row with decreasing offsets gets ST_INVALID and zeroed bytes."""
+        dst = bytes(dst)
+        if _is_device_ragged(msgs):
+            import torch
+            n = max(msgs[1].numel() - 1, 0)
+            m, o = self._ragged_dev(msgs, n)
+            out = torch.empty((n, 65), dtype=torch.uint8, device=msgs[0].device)
+            st = torch.empty(n, dtype=torch.uint8, device=msgs[0].device)
+            a = self._dev_args(out, st)
+            self._check(self._lib.s256_hash_to_curve_varlen_dev(self._ctx, dst, C.c_size_t(len(dst)), m, o, C.c_size_t(n),
+                                                                int(bool(random_oracle)), a[0], a[1], self._stream()),
+                        "hash_to_curve_varlen_dev")
+            return out, st
+        n = len(msgs)
+        flat, offs = self._ragged_host(msgs, n)
+        out = self._out(38, (n, 65))
+        st = self._out(39, n)
+        self._check(self._lib.s256_hash_to_curve_varlen(self._ctx, dst, C.c_size_t(len(dst)), self._hp(flat), self._hp(offs),
+                                                        C.c_size_t(n), int(bool(random_oracle)), self._hp(out), self._hp(st)),
+                    "hash_to_curve_varlen")
         return out, st
 
     def expand_message_xmd(self, dst, msgs, length):

@@ -442,7 +442,7 @@ extern "C" void s256_free(s256_ctx *ctx) {
                         ctx->sink, ctx->msm_counts, ctx->msm_offsets, ctx->msm_cursor, ctx->msm_entries, ctx->msm_flag,
                         ctx->msm_buckets, ctx->msm_win, ctx->msm_acc, ctx->msm_tmp, ctx->msm_cub, ctx->msm_nsl, ctx->msm_sloff,
                         ctx->msm_perm, ctx->msm_hist, ctx->msm_range, ctx->msm_part, ctx->msm_sbkt, ctx->comm_buf, ctx->msm_aff2, ctx->msm_half, ctx->msm_bsum,
-                        ctx->bat, ctx->in_off};
+                        ctx->bat, ctx->in_off, ctx->h2c_dst};
         for (void *p : ptrs)
             if (p) cudaFree(p);
         if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -478,6 +478,7 @@ static int ctx_alloc(s256_ctx *ctx) {
     CK(cudaMalloc(&ctx->out, 65 * cap));
     CK(cudaMalloc(&ctx->st, cap));
     CK(cudaMalloc(&ctx->sink, 16));
+    CK(cudaMalloc(&ctx->h2c_dst, 256));
     return S256_SUCCESS;
 }
 

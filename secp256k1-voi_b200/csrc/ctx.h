@@ -43,6 +43,7 @@ struct s256_ctx {
     size_t in_b_bytes = 0;
     size_t *in_off = nullptr;  // the message offsets of the *_varlen host forms (allocated on first use)
     size_t in_off_count = 0;
+    uint8_t *h2c_dst = nullptr;  // the hash-to-curve DST of the current call (256 bytes, api_h2c.cu)
     unsigned long long *sink = nullptr;
     // MSM scratch (allocated on first use)
     size_t msm_cap = 0;

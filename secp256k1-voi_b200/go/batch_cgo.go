@@ -218,6 +218,28 @@ func (e *Engine) SchnorrSignBatchVarlen(priv32 []byte, msgs [][]byte, aux32 []by
 	return sig64, status, nil
 }
 
+// HashToCurveBatch is h2c.Secp256k1_XMD_SHA256_SSWU_RO (randomOracle) or _NU over messages of any length, one per
+// row, under one domain separation tag: 65 bytes per row (the uncompressed point) and a status byte per row
+// (S256_ST_OK, or S256_ST_IDENTITY with zeroed bytes where the per-item call returns the identity).  An empty dst is
+// an error (errInvalidDomainSep).
+func (e *Engine) HashToCurveBatch(dst []byte, msgs [][]byte, randomOracle bool) ([]byte, []byte, error) {
+	if len(dst) == 0 {
+		return nil, nil, errors.New("secp256k1/secec/h2c: invalid domain separator")
+	}
+	n := len(msgs)
+	flat, offs := raggedRows(msgs)
+	ro := C.int(0)
+	if randomOracle {
+		ro = 1
+	}
+	out65, status := make([]byte, 65*n), make([]byte, n)
+	if err := e.err(C.s256_hash_to_curve_varlen(e.ctx, ptr(dst), C.size_t(len(dst)), ptr(flat), &offs[0], C.size_t(n), ro,
+		ptr(out65), ptr(status))); err != nil {
+		return nil, nil, err
+	}
+	return out65, status, nil
+}
+
 // ScalarBaseMultBatch is Point.ScalarBaseMult + UncompressedBytes (constant time).
 func (e *Engine) ScalarBaseMultBatch(scalars []*secp256k1.Scalar) ([]*secp256k1.Point, error) {
 	n := len(scalars)

@@ -923,6 +923,17 @@ inline Point Secp256k1_XMD_SHA256_SSWU_NU(const uint8_t *dst, size_t dst_len, co
                                           Engine &e = Engine::Default()) {
     return Secp256k1_XMD_SHA256_SSWU(false, dst, dst_len, msg, msg_len, e);
 }
+// Secp256k1_XMD_SHA256_SSWU_RO (random_oracle) or _NU over messages of any length, one per row (msgs.size() rows)
+// under one DST: out65 gets the uncompressed point of each row and status S256_ST_OK, or 65 zero bytes and
+// S256_ST_IDENTITY where the per-item call returns the identity.
+inline void HashToCurveBatch(const std::vector<uint8_t> &dst, const std::vector<std::vector<uint8_t>> &msgs, bool random_oracle,
+                             uint8_t *out65, uint8_t *status, Engine &e = Engine::Default()) {
+    if (dst.empty()) throw Error("secp256k1/secec/h2c: invalid domain separator");
+    bitcoin::detail::RaggedRows r(msgs);
+    e.check(s256_hash_to_curve_varlen(e.ctx(), dst.data(), dst.size(), r.data(), r.offsets.data(), msgs.size(),
+                                      random_oracle ? 1 : 0, out65, status),
+            "HashToCurveBatch");
+}
 }  // namespace h2c
 }  // namespace secec
 }  // namespace secp256k1
